@@ -85,6 +85,11 @@ class Workload:
     def resident(self, first, n, device):
         return [s.on_device(first, n, device=device) for s in self.specs()]
 
+    def outputs(self, table=None):
+        """What one pass hands its caller: groups of named arrays (device tensors or host arrays), the arrays of a group
+        sharing their rows (one per unit or per table entry).  `table`: the merged table of N > 1 GPUs, else the plan's."""
+        raise NotImplementedError
+
     @staticmethod
     def same(a, b):
         return len(a) == len(b) and all(np.array_equal(np.asarray(x), np.asarray(y)) for x, y in zip(a, b))
@@ -131,6 +136,9 @@ class SingleWorkload(Workload):
 
     def result(self):
         return [self.counts.cpu().numpy()]
+
+    def outputs(self, table=None):
+        return [{"counts": self.counts}, {"index": self.index}]
 
     def matched(self):
         return int(self.counts.sum().item())
@@ -202,6 +210,9 @@ class DualWorkload(Workload):
     def result(self):
         return [self.counts.cpu().numpy()]
 
+    def outputs(self, table=None):
+        return [{"counts": self.counts}, {"index": self.index}]
+
     def matched(self):
         return int(self.counts.sum().item())
 
@@ -261,6 +272,10 @@ class ComboWorkload(Workload):
     def result(self):
         keys, freq = self.plan.harvest()
         return [keys, freq]
+
+    def outputs(self, table=None):
+        keys, freq = table or self.plan.harvest()
+        return [{"keys": keys, "freq": freq}, {"pairs": self.pairs.view(-1, 2)}]
 
     def matched(self):
         return int(self.plan.harvest()[1].sum())
@@ -325,6 +340,12 @@ class RandomWorkload(Workload):
         seqs, freq = self.plan.harvest()
         return [seqs, freq]
 
+    def outputs(self, table=None):
+        seqs, freq = table or self.plan.harvest()
+        # the barcodes (fixed-width bytes) as one row of character codes each
+        codes = np.frombuffer(seqs.tobytes(), dtype=np.uint8).reshape(len(seqs), seqs.dtype.itemsize)
+        return [{"barcodes": codes, "freq": freq}, {"index": self.index}]
+
     def matched(self):
         return int(self.plan.harvest()[1].sum())
 
@@ -352,6 +373,29 @@ def make_workload(number):
     if number in (1, 2):
         return SingleWorkload(number)
     return {3: DualWorkload, 4: ComboWorkload, 5: RandomWorkload}[number]()
+
+
+DUMP_VALUES = 1 << 20   # per array: 8 MB in float64, so at most 32 MB for the (up to three) arrays of a workload
+
+
+def dump_outputs(wl, out_dir, table=None):
+    """--dump-outputs: writes the arrays of the last timed pass as <out_dir>/<name>.npy in float64 (all of them hold integers
+    below 2**53, so the values are exact).  A group of arrays whose widest holds more than DUMP_VALUES values keeps one
+    sample of rows, drawn with the benchmark's seed, for all its arrays: the same rows from run to run, so that two builds
+    can be compared output for output, and row i of one array belongs with row i of the others."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for group in wl.outputs(table):
+        rows = len(next(iter(group.values())))
+        keep = max(1, DUMP_VALUES // max(max(1, int(np.prod(a.shape[1:]))) for a in group.values()))
+        rows_kept = np.sort(np.random.default_rng(SEED).choice(rows, keep, replace=False)) if rows > keep else None
+        for name, arr in group.items():
+            assert len(arr) == rows, "arrays of one group share their rows"
+            if rows_kept is not None:
+                arr = arr[torch.from_numpy(rows_kept).to(arr.device)] if torch.is_tensor(arr) else arr[rows_kept]
+            if torch.is_tensor(arr):
+                arr = arr.cpu().numpy()
+            np.save(os.path.join(out_dir, name + ".npy"), np.asarray(arr, dtype=np.float64))
 
 
 # =====================================================================================================================
@@ -660,7 +704,12 @@ def main():
     ap.add_argument("--reads", type=int, default=0, help="units resident per GPU (weak) or in total (strong); default: the config's size")
     ap.add_argument("--e2e-reads", dest="e2e_units", type=int, default=0, help="units per end-to-end step (host FASTQ text)")
     ap.add_argument("--cpu-reads", dest="cpu_units", type=int, default=0, help="units in the bounded CPU-baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64; counts and tables "
+                         "merged over the GPUs, per-unit outcomes of rank 0's units; larger arrays as a fixed seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -778,6 +827,10 @@ def main():
         elapsed = e0.elapsed_time(e1)
     gpu_launches = rcpp.kernel_launches(local_rank) - launches_before
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # N > 1: counts were summed over the ranks in place; sparse tables were merged into the exchange (on rank 0)
+        merged = exchange.result() if exchange is not None and exchange.kind == "table" else None
+        dump_outputs(wl, args.dump_outputs, merged)
     elapsed_ms = torch.tensor([elapsed], device=dev)
     if world > 1:
         dist.all_reduce(elapsed_ms, op=dist.ReduceOp.MAX)

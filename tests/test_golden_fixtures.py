@@ -28,6 +28,19 @@ def _sorted_table(seqs, freq):
     return [list(seqs)[i] for i in order], np.asarray(freq)[order]
 
 
+def _pair_table(pairs):
+    """Per-read (or per-pair) combinations -> the table the reference reports: the distinct matched rows with their counts."""
+    pairs = np.asarray(pairs).reshape(-1, 2)
+    return np.unique(pairs[(pairs >= 0).all(axis=1)], axis=0, return_counts=True)
+
+
+def _eq_table(got_keys, got_freq, c, what):
+    want_keys = np.asarray(c["keys"]).reshape(len(c["freq"]), -1)
+    order = np.lexsort(want_keys.T[::-1]) if len(want_keys) else np.zeros(0, dtype=np.int64)
+    _eq(got_keys.reshape(len(got_freq), -1), want_keys[order], what + " (combinations)")
+    _eq(got_freq, np.asarray(c["freq"])[order], what + " (frequencies)")
+
+
 def check(engine, c):
     kind = c["kind"]
     if kind == "single":
@@ -50,6 +63,9 @@ def check(engine, c):
         _eq(np.asarray(keys).reshape(len(freq), -1), np.asarray(c["keys"]).reshape(len(c["freq"]), -1), "combinations")
         _eq(freq, c["freq"], "frequencies")
         assert total == c["total"]
+        trace = engine.trace_combo_single(fastq(c["reads"]), c["template"], c["strand"], c["pool1"], c["pool2"], c["mismatches"],
+                                          c["use_first"])
+        _eq_table(*_pair_table(trace), c, "per-read combinations")
     elif kind == "dual_single_end":
         res = engine.count_dual_single_end(fastq(c["reads"]), c["template"], c["pools"], c["strand"], c["mismatches"], c["use_first"],
                                            c["diagnostics"])
@@ -58,6 +74,9 @@ def check(engine, c):
         if c["diagnostics"]:
             _eq(np.asarray(res[2]).reshape(len(res[3]), -1), np.asarray(c["keys"]).reshape(len(c["freq"]), -1), "invalid combinations")
             _eq(res[3], c["freq"], "invalid frequencies")
+        index = np.asarray(engine.trace_dual_single_end(fastq(c["reads"]), c["template"], c["pools"], c["strand"], c["mismatches"],
+                                                        c["use_first"]))
+        _eq(np.bincount(index[index >= 0], minlength=len(c["counts"])), c["counts"], "counts of the per-read trace")
     elif kind == "dual":
         f1, f2 = fastq(c["reads1"]), fastq(c["reads2"])
         args = (f1, c["template1"], c["reverse1"], c["mismatches1"], c["pool1"], f2, c["template2"], c["reverse2"], c["mismatches2"],
@@ -83,6 +102,11 @@ def check(engine, c):
         _eq(np.asarray(keys).reshape(len(freq), -1), np.asarray(c["keys"]).reshape(len(c["freq"]), -1), "combinations")
         _eq(freq, c["freq"], "frequencies")
         assert (total, b1, b2) == (c["total"], c["barcode1_only"], c["barcode2_only"])
+        combo, code = engine.trace_combo_paired(f1, c["template1"], c["reverse1"], c["mismatches1"], c["pool1"], f2, c["template2"],
+                                                c["reverse2"], c["mismatches2"], c["pool2"], c["randomized"], c["use_first"])
+        _eq_table(*_pair_table(combo), c, "per-pair combinations")
+        code = np.asarray(code)
+        assert (int((code == 2).sum()), int((code == 3).sum())) == (c["barcode1_only"], c["barcode2_only"])
     elif kind == "match":
         if "error" in c:
             with pytest.raises(Exception):
@@ -105,6 +129,17 @@ def test_fixture_is_complete():
 @pytest.mark.parametrize("case", CASES, ids=lambda c: c["name"])
 def test_port_matches_reference_fixture(port, case):
     check(port, case)
+
+
+@pytest.mark.parametrize("case", [c for c in CASES if c["kind"] == "match" and "error" not in c], ids=lambda c: c["name"])
+def test_port_search_any_matches_reference_fixture(port, case):
+    """The restatement's search with a cap per query (the yardstick of tests/test_gpu_segmented.py), every cap set to the
+    substitutions of the reference's matchBarcodes run, finds what that run found."""
+    caps = np.full(len(case["seqs"]), case["substitutions"], dtype=np.int32)
+    index, mm = port.search_any(case["seqs"], caps, case["choices"], case["substitutions"], case["reverse"])
+    index = np.where(index >= 0, index, -1)   # no hit (-1) and an ambiguous one (-2) are both NA in matchBarcodes
+    _eq(index, case["index"], "index")
+    _eq(np.where(np.asarray(index) >= 0, mm, -1), np.where(np.asarray(case["index"]) >= 0, np.asarray(case["mm"]), -1), "mismatches")
 
 
 @pytest.mark.gpu

@@ -8,9 +8,9 @@ from fastq_cases import GOOD, BAD
 
 
 @pytest.mark.parametrize("name", sorted(GOOD))
-def test_good(kref, port, name):
+def test_good(compiled_reference, port, name):
     data = GOOD[name]
-    assert kref.parse(data) == port.parse(data)
+    assert compiled_reference.parse(data) == port.parse(data)
 
 
 def test_expected_shapes(kref):

@@ -11,5 +11,5 @@ def test_port_golden(port, case):
 
 
 @pytest.mark.parametrize("case", golden_cases.ALL, ids=lambda f: f.__name__)
-def test_reference_golden(kref, case):
-    case(kref)
+def test_reference_golden(compiled_reference, case):
+    case(compiled_reference)
