@@ -52,9 +52,11 @@ enum { SCG_STRAND_ORIGINAL = 0, SCG_STRAND_REVERSE = 1, SCG_STRAND_BOTH = 2 };
 /* ---- context ------------------------------------------------------------------------ */
 int scg_ctx_create(scg_ctx** out, int device);       /* device = CUDA ordinal; lazy init */
 /* One context over SEVERAL devices (the reference runs its threads inside one call, inst/include/kaori/process_data.hpp:131-177;
- * this is the same for GPUs): scg_count_single cuts the text of a raw or block-gzip file (or of a memory buffer) at record
- * boundaries into one part per device, and the scg_count_*_many calls deal their files to the devices.  Every other entry point
- * runs on the first device.  Inputs that cannot be cut (plain gzip streams, small files) are read by the first device alone. */
+ * this is the same for GPUs): the single-end entry points scg_count_single, scg_count_combo_single, scg_count_dual_single_end and
+ * scg_count_random cut the text of a raw or block-gzip file (or of a memory buffer) at record boundaries into one part per
+ * device, and merge the parts' results into exactly what a context of one device returns; the scg_count_*_many calls deal
+ * their files to the devices.  Inputs that cannot be cut (plain gzip streams, small files) are read by one device alone.
+ * The paired-input entry points (scg_count_dual, scg_count_combo_paired, scg_count_single_paired) run on the first device. */
 int scg_ctx_create_multi(scg_ctx** out, const int* devices, int n_devices);
 int scg_ctx_devices(const scg_ctx* ctx);
 void scg_ctx_destroy(scg_ctx* ctx);

@@ -210,6 +210,8 @@ struct CountTable {
 // device-side helpers on sorted tables (runners_random.cu)
 void render_barcodes(Context& ctx, const SortedTable& t, DeviceBuffer& strings, DeviceBuffer& freq);   // rows * key_len chars, int32 freq
 void render_combinations(Context& ctx, const SortedTable& t, DeviceBuffer& keys, DeviceBuffer& freq);  // rows * 2 int32 (first, second), int32 freq
+// out = t rendered (barcodes when t.key_len > 0, combinations otherwise) and left on the device for scg_result_copy_table
+void device_table_result(Context& ctx, const SortedTable& t, scg_result& out);
 // c = sorted merge of a and b with the counts of equal keys added (a and b sorted ascending, keys unique within each)
 void merge_sorted_tables(Context& ctx, const SortedTable& a, const SortedTable& b, SortedTable& c);
 

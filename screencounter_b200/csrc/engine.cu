@@ -221,10 +221,10 @@ int Context::grid_for(long long ntiles) const {
 void Context::finish_timing() {
     char buf[512];
     std::snprintf(buf, sizeof buf,
-                  "{\"parse_s\": %.6f, \"pack_s\": %.6f, \"h2d_s\": %.6f, \"device_s\": %.6f, \"setup_s\": %.6f, \"harvest_s\": %.6f, \"total_s\": %.6f, "
-                  "\"reads\": %lld, \"bytes_h2d\": %lld, \"launches\": %lld, \"reader\": \"%s\", \"kernel\": \"",
-                  timing.parse_s, timing.pack_s, timing.h2d_s, timing.device_s, timing.setup_s, timing.harvest_s, timing.total_s, timing.reads, timing.bytes_h2d,
-                  timing.launches, timing.reader.c_str());
+                  "{\"parse_s\": %.6f, \"pack_s\": %.6f, \"h2d_s\": %.6f, \"device_s\": %.6f, \"setup_s\": %.6f, \"harvest_s\": %.6f, \"merge_s\": %.6f, "
+                  "\"total_s\": %.6f, \"reads\": %lld, \"bytes_h2d\": %lld, \"launches\": %lld, \"reader\": \"%s\", \"kernel\": \"",
+                  timing.parse_s, timing.pack_s, timing.h2d_s, timing.device_s, timing.setup_s, timing.harvest_s, timing.merge_s, timing.total_s,
+                  timing.reads, timing.bytes_h2d, timing.launches, timing.reader.c_str());
     timing_json = buf;
     for (char ch : kernel_note) {
         if (ch == '"' || ch == '\\' || (unsigned char)ch < 0x20) ch = ' ';

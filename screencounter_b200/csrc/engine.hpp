@@ -56,6 +56,7 @@ struct Timing {
     double parse_s = 0, pack_s = 0, h2d_s = 0, device_s = 0, total_s = 0;
     double harvest_s = 0; // variable-size results (combination / random-barcode tables) sorted, downloaded and rendered
     double setup_s = 0;   // library tables built + uploaded, kernels specialised (zero when the context had them cached)
+    double merge_s = 0;   // a call cut over several devices: the parts' results merged on the first device
     long long reads = 0, bytes_h2d = 0, launches = 0;
     std::string reader = "host";   // which FASTQ reader fed the call: the host parser/packer or the device one (ingest.hpp)
 };

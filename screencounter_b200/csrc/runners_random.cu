@@ -302,6 +302,20 @@ void render_combinations(Context& ctx, const SortedTable& t, DeviceBuffer& keys,
     ++ctx.launches;
 }
 
+void device_table_result(Context& ctx, const SortedTable& t, scg_result& out) {
+    if (t.key_len > 0) {
+        out.width = t.key_len;
+        render_barcodes(ctx, t, out.d_strings, out.d_freq);
+    } else {
+        out.width = 2;
+        render_combinations(ctx, t, out.d_keys, out.d_freq);
+    }
+    SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    out.on_device = true;
+    out.device = ctx.device;
+    out.d_rows = t.rows;
+}
+
 // Merge of two sorted tables (the device-side reduce() of handlers/RandomBarcodeSingleEnd.hpp:197-207 and of the
 // combinations' append + sort, handlers/CombinatorialBarcodesSingleEnd.hpp:268-305): every row finds its place in the
 // output by a binary search in the OTHER table -- rank = own index + rows of the other table that sort before it, minus
@@ -524,14 +538,9 @@ void ComboTally::sorted(Context& ctx, SortedTable& out) {
 // rows sorted ascending by (first, second), one frequency per distinct combination.  Sorted and rendered on the device;
 // the table stays there until scg_result_copy_table copies it into the caller's arrays.
 void ComboTally::harvest(Context& ctx, scg_result& out) {
-    out.width = 2;
     SortedTable t;
     sorted(ctx, t);
-    render_combinations(ctx, t, out.d_keys, out.d_freq);
-    SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-    out.on_device = true;
-    out.device = ctx.device;
-    out.d_rows = t.rows;
+    device_table_result(ctx, t, out);
 }
 
 namespace {
@@ -572,164 +581,162 @@ extern "C" {
 
 namespace scg {
 
-// countRandomBarcodes over one input on one device.  With want_sorted set, a table that can stay on the device as sorted
-// 64-bit keys (barcodes of up to 21 bases, no key taken from raw read text) is handed over there and *table stays null:
-// what the many-files call unites on the device (runners_multi.cu).
-void count_random_core(scg_ctx* ctx, const scg_source* src, const char* constant, int strand, int mismatches, int use_first,
-                       int nthreads, SortedTable* want_sorted, scg_result** table, int32_t* total) {
-    {
-        Context& c = ctx->impl;
-        const double t_start = now_s();
-        c.timing = Timing();
-        Source source(src);
-        RandomMatcher m;
-        m.prepare(constant, strand, mismatches, use_first != 0);
-        const TemplateSpec& tmpl = m.tmpl;
-        const int key_len = m.key_len;
-        const bool wide = m.wide;
+// countRandomBarcodes over one reader.  Barcodes of up to 21 bases, none taken from raw read text, stay on the device as a
+// sorted table (rank-coded, text order); any other result is rendered on the host.
+void count_random_reader(Context& c, FastqReader* reader, const RandomMatcher& m, int nthreads, SparseCounts& result) {
+    const TemplateSpec& tmpl = m.tmpl;
+    const int key_len = m.key_len;
+    const bool wide = m.wide;
 
-        c.ensure_ready();
-        CountTable tab;
-        tab.init(c, wide, wide ? (1u << 20) : (1u << 23));   // 8 M slots (128 MB) to start with: a few million distinct barcodes need no rehash
-        DeviceBuffer d_odd_out, d_odd_count;
-        d_odd_count.alloc(sizeof(unsigned long long), true);
-        std::map<std::string, int> extra;   // keys of reads that need their raw text
+    c.ensure_ready();
+    CountTable tab;
+    tab.init(c, wide, wide ? (1u << 20) : (1u << 23));   // 8 M slots (128 MB) to start with: a few million distinct barcodes need no rehash
+    DeviceBuffer d_odd_out, d_odd_count;
+    d_odd_count.alloc(sizeof(unsigned long long), true);
+    std::map<std::string, int> extra;   // keys of reads that need their raw text
 
-        ReadPipeline pipe(c, source.reader.get(), nullptr, nthreads, true);
-        ReadPipeline::Batch b;
-        long long nreads = 0;
-        std::vector<OddOutcome> odd_host;
-        while (pipe.next(b)) {
-            {
-                const double t0 = now_s();
-                tab.ensure(c, b.n);
-                c.timing.setup_s += now_s() - t0;
-            }
-            // reads flagged odd get their outcome reported back; the device-side reader only knows on the device how many
-            // there are (count_odd < 0), so room is made for all
-            const long long nodd_host = pipe.count_odd(b);
-            const long long nodd = nodd_host < 0 ? b.n : nodd_host;
-            d_odd_out.reserve((size_t)std::max<long long>(nodd, 1) * sizeof(OddOutcome));
-            SCG_CUDA_CHECK(cudaMemsetAsync(d_odd_count.ptr, 0, sizeof(unsigned long long), c.stream));
-            launch_random(c, b.reads1, m, tab, b.odd1, d_odd_out.as<OddOutcome>(), d_odd_count.as<unsigned long long>(), nullptr, c.stream);
-            pipe.submitted(b);
-            if (nodd > 0) {
-                // reads holding lower-case letters or symbols other than N: the device decided where the
-                // barcode sits, the host renders it from the raw read text exactly as the reference would
-                unsigned long long got = 0;
-                SCG_CUDA_CHECK(cudaMemcpyAsync(&got, d_odd_count.ptr, sizeof got, cudaMemcpyDeviceToHost, c.stream));
+    ReadPipeline pipe(c, reader, nullptr, nthreads, true);
+    ReadPipeline::Batch b;
+    long long nreads = 0;
+    std::vector<OddOutcome> odd_host;
+    while (pipe.next(b)) {
+        {
+            const double t0 = now_s();
+            tab.ensure(c, b.n);
+            c.timing.setup_s += now_s() - t0;
+        }
+        // reads flagged odd get their outcome reported back; the device-side reader only knows on the device how many
+        // there are (count_odd < 0), so room is made for all
+        const long long nodd_host = pipe.count_odd(b);
+        const long long nodd = nodd_host < 0 ? b.n : nodd_host;
+        d_odd_out.reserve((size_t)std::max<long long>(nodd, 1) * sizeof(OddOutcome));
+        SCG_CUDA_CHECK(cudaMemsetAsync(d_odd_count.ptr, 0, sizeof(unsigned long long), c.stream));
+        launch_random(c, b.reads1, m, tab, b.odd1, d_odd_out.as<OddOutcome>(), d_odd_count.as<unsigned long long>(), nullptr, c.stream);
+        pipe.submitted(b);
+        if (nodd > 0) {
+            // reads holding lower-case letters or symbols other than N: the device decided where the
+            // barcode sits, the host renders it from the raw read text exactly as the reference would
+            unsigned long long got = 0;
+            SCG_CUDA_CHECK(cudaMemcpyAsync(&got, d_odd_count.ptr, sizeof got, cudaMemcpyDeviceToHost, c.stream));
+            SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
+            odd_host.resize(got);
+            if (got) {
+                SCG_CUDA_CHECK(cudaMemcpyAsync(odd_host.data(), d_odd_out.ptr, got * sizeof(OddOutcome), cudaMemcpyDeviceToHost, c.stream));
                 SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
-                odd_host.resize(got);
-                if (got) {
-                    SCG_CUDA_CHECK(cudaMemcpyAsync(odd_host.data(), d_odd_out.ptr, got * sizeof(OddOutcome), cudaMemcpyDeviceToHost, c.stream));
-                    SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
-                }
-                std::sort(odd_host.begin(), odd_host.end(), [](const OddOutcome& x, const OddOutcome& y) { return x.read < y.read; });
-                std::string key(key_len, ' ');
-                std::string seq;
-                for (const auto& o : odd_host) {
-                    pipe.raw_read(b, (long long)o.read, seq);
-                    const char* start = seq.data() + o.position + tmpl.fwd_regions[0].start;
-                    if (!o.reverse) {  // forward_match: raw characters (handlers/RandomBarcodeSingleEnd.hpp:93-104)
-                        key.assign(start, key_len);
-                    } else {  // reverse_match: complement_base<true> (:106-120, utils.hpp:41-62)
-                        for (int j = 0; j < key_len; ++j) {
-                            const char ch = start[key_len - j - 1];
-                            char out;
-                            switch (ch) {
-                                case 'A': case 'a': out = 'T'; break;
-                                case 'C': case 'c': out = 'G'; break;
-                                case 'G': case 'g': out = 'C'; break;
-                                case 'T': case 't': out = 'A'; break;
-                                case 'N': case 'n': out = 'N'; break;
-                                default: throw Error(std::string("cannot complement unknown base '") + ch + "'");
-                            }
-                            key[j] = out;
+            }
+            std::sort(odd_host.begin(), odd_host.end(), [](const OddOutcome& x, const OddOutcome& y) { return x.read < y.read; });
+            std::string key(key_len, ' ');
+            std::string seq;
+            for (const auto& o : odd_host) {
+                pipe.raw_read(b, (long long)o.read, seq);
+                const char* start = seq.data() + o.position + tmpl.fwd_regions[0].start;
+                if (!o.reverse) {  // forward_match: raw characters (handlers/RandomBarcodeSingleEnd.hpp:93-104)
+                    key.assign(start, key_len);
+                } else {  // reverse_match: complement_base<true> (:106-120, utils.hpp:41-62)
+                    for (int j = 0; j < key_len; ++j) {
+                        const char ch = start[key_len - j - 1];
+                        char out;
+                        switch (ch) {
+                            case 'A': case 'a': out = 'T'; break;
+                            case 'C': case 'c': out = 'G'; break;
+                            case 'G': case 'g': out = 'C'; break;
+                            case 'T': case 't': out = 'A'; break;
+                            case 'N': case 'n': out = 'N'; break;
+                            default: throw Error(std::string("cannot complement unknown base '") + ch + "'");
                         }
+                        key[j] = out;
                     }
-                    ++extra[key];
                 }
-            }
-            nreads += b.n;
-        }
-        const double t_harvest = now_s();
-        auto* r = new scg_result;
-        std::unique_ptr<scg_result> guard(r);
-        r->width = key_len;
-        if (!wide) {
-            // barcodes of up to 21 bases: sorted as text ON THE DEVICE (radix sort of rank-coded keys)
-            SortedTable sorted;
-            tab.sorted(c, key_len, sorted);
-            if (extra.empty() && want_sorted) {
-                *want_sorted = std::move(sorted);
-                guard.reset();
-            } else if (extra.empty()) {
-                // ... rendered there too, and left there: scg_result_copy_table copies the finished table straight into the
-                // caller's arrays (one device-to-host copy, no host image in between)
-                render_barcodes(c, sorted, r->d_strings, r->d_freq);
-                SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
-                r->on_device = true;
-                r->device = c.device;
-                r->d_rows = sorted.rows;
-            } else {
-                // a few keys came from raw read text (lower case, IUPAC letters): merged on the host in text order
-                const size_t n = sorted.rows;
-                std::vector<unsigned long long> order_keys(n);
-                std::vector<uint32_t> cnt(n);
-                if (n) {
-                    SCG_CUDA_CHECK(cudaMemcpyAsync(order_keys.data(), sorted.keys.ptr, n * 8, cudaMemcpyDeviceToHost, c.stream));
-                    SCG_CUDA_CHECK(cudaMemcpyAsync(cnt.data(), sorted.counts.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
-                    SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
-                }
-                auto render = [&](unsigned long long k, char* out) {
-                    for (int b = key_len - 1; b >= 0; --b) {
-                        out[b] = "ACGNT"[k & 7ull];
-                        k >>= 3;
-                    }
-                };
-                r->strings.reserve((n + extra.size()) * (size_t)key_len);
-                r->freq.reserve(n + extra.size());
-                std::string cur(key_len, ' ');
-                auto it = extra.begin();
-                auto emit = [&](const std::string& k, int f) {
-                    r->strings.insert(r->strings.end(), k.begin(), k.end());
-                    r->freq.push_back(f);
-                };
-                for (size_t i = 0; i < n; ++i) {
-                    render(order_keys[i], &cur[0]);
-                    while (it != extra.end() && it->first < cur) {
-                        emit(it->first, it->second);
-                        ++it;
-                    }
-                    int f = (int)cnt[i];
-                    if (it != extra.end() && it->first == cur) {
-                        f += it->second;
-                        ++it;
-                    }
-                    emit(cur, f);
-                }
-                for (; it != extra.end(); ++it) emit(it->first, it->second);
-            }
-        } else {
-            std::vector<unsigned long long> lo, hi;
-            std::vector<uint32_t> cnt;
-            tab.download(c, lo, hi, cnt);
-            std::map<std::string, int> merged(std::move(extra));
-            for (size_t i = 0; i < lo.size(); ++i) merged[decode_key(lo[i], hi[i], key_len, wide)] += (int)cnt[i];
-            r->strings.reserve(merged.size() * (size_t)key_len);
-            r->freq.reserve(merged.size());
-            for (const auto& kv : merged) {  // std::map iterates in byte order = R's order(sequences) for ACGTN text
-                r->strings.insert(r->strings.end(), kv.first.begin(), kv.first.end());
-                r->freq.push_back(kv.second);
+                ++extra[key];
             }
         }
-        c.timing.harvest_s = now_s() - t_harvest;
-        *table = guard.release();
-        *total = (int32_t)nreads;
-        c.timing.parse_s = source.reader->parse_seconds();
-        c.timing.total_s = now_s() - t_start;
-        c.finish_timing();
+        nreads += b.n;
     }
+    const double t_harvest = now_s();
+    result.reads = nreads;
+    std::unique_ptr<scg_result> r(new scg_result);
+    r->width = key_len;
+    if (!wide) {
+        // barcodes of up to 21 bases: sorted as text ON THE DEVICE (radix sort of rank-coded keys)
+        SortedTable sorted;
+        tab.sorted(c, key_len, sorted);
+        if (extra.empty()) {
+            result.table = std::move(sorted);
+            c.timing.harvest_s = now_s() - t_harvest;
+            return;
+        }
+        {
+            // a few keys came from raw read text (lower case, IUPAC letters): merged on the host in text order
+            const size_t n = sorted.rows;
+            std::vector<unsigned long long> order_keys(n);
+            std::vector<uint32_t> cnt(n);
+            if (n) {
+                SCG_CUDA_CHECK(cudaMemcpyAsync(order_keys.data(), sorted.keys.ptr, n * 8, cudaMemcpyDeviceToHost, c.stream));
+                SCG_CUDA_CHECK(cudaMemcpyAsync(cnt.data(), sorted.counts.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+                SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
+            }
+            auto render = [&](unsigned long long k, char* out) {
+                for (int b = key_len - 1; b >= 0; --b) {
+                    out[b] = "ACGNT"[k & 7ull];
+                    k >>= 3;
+                }
+            };
+            r->strings.reserve((n + extra.size()) * (size_t)key_len);
+            r->freq.reserve(n + extra.size());
+            std::string cur(key_len, ' ');
+            auto it = extra.begin();
+            auto emit = [&](const std::string& k, int f) {
+                r->strings.insert(r->strings.end(), k.begin(), k.end());
+                r->freq.push_back(f);
+            };
+            for (size_t i = 0; i < n; ++i) {
+                render(order_keys[i], &cur[0]);
+                while (it != extra.end() && it->first < cur) {
+                    emit(it->first, it->second);
+                    ++it;
+                }
+                int f = (int)cnt[i];
+                if (it != extra.end() && it->first == cur) {
+                    f += it->second;
+                    ++it;
+                }
+                emit(cur, f);
+            }
+            for (; it != extra.end(); ++it) emit(it->first, it->second);
+        }
+    } else {
+        std::vector<unsigned long long> lo, hi;
+        std::vector<uint32_t> cnt;
+        tab.download(c, lo, hi, cnt);
+        std::map<std::string, int> merged(std::move(extra));
+        for (size_t i = 0; i < lo.size(); ++i) merged[decode_key(lo[i], hi[i], key_len, wide)] += (int)cnt[i];
+        r->strings.reserve(merged.size() * (size_t)key_len);
+        r->freq.reserve(merged.size());
+        for (const auto& kv : merged) {  // std::map iterates in byte order = R's order(sequences) for ACGTN text
+            r->strings.insert(r->strings.end(), kv.first.begin(), kv.first.end());
+            r->freq.push_back(kv.second);
+        }
+    }
+    c.timing.harvest_s = now_s() - t_harvest;
+    result.rendered = std::move(r);
+}
+
+void count_random_file(scg_ctx* ctx, const scg_source* src, const char* constant, int strand, int mismatches, int use_first, int nthreads,
+                       bool split_over_devices, SparseCounts& out) {
+    Context& c = ctx->impl;
+    const double t_start = now_s();
+    c.timing = Timing();
+    Source source(src);
+    RandomMatcher m;
+    m.prepare(constant, strand, mismatches, use_first != 0);
+    c.ensure_ready();
+    if (!(split_over_devices && !ctx->peers.empty() &&
+          count_random_multi(ctx, *source.reader, constant, strand, mismatches, use_first, nthreads, out))) {
+        count_random_reader(c, source.reader.get(), m, nthreads, out);
+        c.timing.parse_s = source.reader->parse_seconds();
+    }
+    c.timing.total_s = now_s() - t_start;
+    c.finish_timing();
 }
 
 } // namespace scg
@@ -738,7 +745,18 @@ extern "C" {
 
 int scg_count_random(scg_ctx* ctx, const scg_source* src, const char* constant, int strand, int mismatches, int use_first,
                      int nthreads, scg_result** table, int32_t* total) {
-    return guarded(ctx, [&] { count_random_core(ctx, src, constant, strand, mismatches, use_first, nthreads, nullptr, table, total); });
+    return guarded(ctx, [&] {
+        SparseCounts counts;
+        count_random_file(ctx, src, constant, strand, mismatches, use_first, nthreads, true, counts);
+        if (!counts.rendered) {
+            // the table was sorted on the device: rendered there too, and left there (scg_result_copy_table copies the finished
+            // table straight into the caller's arrays, no host image in between)
+            counts.rendered.reset(new scg_result);
+            device_table_result(ctx->impl, counts.table, *counts.rendered);
+        }
+        *table = counts.rendered.release();
+        *total = (int32_t)counts.reads;
+    });
 }
 
 } // extern "C"
