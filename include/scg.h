@@ -251,18 +251,27 @@ int scg_plan_harvest(scg_plan* plan, scg_result** table);
 /* Sparse results as sorted tables ON THE DEVICE: what GPUs exchange when the table of one file (or of several files) is
  * merged across them -- the device-side counterpart of the reference's reduce() for random barcodes
  * (inst/include/kaori/handlers/RandomBarcodeSingleEnd.hpp:197-207) and of the append + sort of combinations
- * (handlers/CombinatorialBarcodesSingleEnd.hpp:268-305, R/combineComboCounts.R:31-57).  keys: unsigned 64-bit, ascending,
- * unique -- combinations as first << 32 | second, random barcodes as three bits per base in text order (A < C < G < N < T),
- * first base most significant; counts: unsigned 32-bit.  key_len > 0 marks random barcodes of that length.
+ * (handlers/CombinatorialBarcodesSingleEnd.hpp:268-305, R/combineComboCounts.R:31-57).  keys (scg_table_keys): rows of
+ * scg_table_key_words(t) unsigned 64-bit words each, row-major, ascending by (word 0, word 1), unique --
+ *   combinations               one word, first << 32 | second;
+ *   random barcodes <= 21 bases  one word, three bits per base in text order (A=0 < C=1 < G=2 < N=3 < T=4), first base most
+ *                              significant;
+ *   random barcodes 22..42     two words: word 0 = bases 0..20 as above (the one-word key of the first 21 bases), word 1 =
+ *                              bases 21..key_len-1 in the same convention.
+ * Every word is below 2^63, so signed 64-bit views keep the order.  counts: unsigned 32-bit, one per row.  key_len > 0 marks
+ * random barcodes of that length; the number of words follows from it (two when key_len > 21).
  *   scg_plan_sorted_table   the plan's tally, sorted (synchronises the device)
  *   scg_plan_dense_tally    combinations tallied in a dense n1 x n2 matrix: its device address (else *d_matrix = NULL)
- *   scg_table_from_device   a table from device arrays the caller owns (copied), e.g. rows received from another GPU
- *   scg_table_merge         sorted union of two tables, counts of equal keys added
+ *   scg_table_key_words     64-bit words per row of the table's keys (1 or 2)
+ *   scg_table_from_device   a table from device arrays the caller owns (copied: rows x words keys, rows counts), e.g. rows
+ *                           received from another GPU
+ *   scg_table_merge         sorted union of two tables, counts of equal keys added; tables of different key_len are refused
  *   scg_table_render        the table as the file-level calls return it (rows stay on the device until copied) */
 int scg_plan_sorted_table(scg_plan* plan, scg_table** out);
 int scg_plan_dense_tally(scg_plan* plan, void** d_matrix, long long* cells);
 long long scg_table_rows(const scg_table* t);
 int scg_table_key_len(const scg_table* t);
+int scg_table_key_words(const scg_table* t);
 void* scg_table_keys(const scg_table* t);
 void* scg_table_counts(const scg_table* t);
 int scg_table_from_device(scg_ctx* ctx, const void* d_keys, const void* d_counts, long long rows, int key_len, scg_table** out);

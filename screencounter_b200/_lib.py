@@ -75,6 +75,7 @@ def lib():
         L.scg_table_rows.restype = C.c_longlong
         L.scg_table_rows.argtypes = [C.c_void_p]
         L.scg_table_key_len.argtypes = [C.c_void_p]
+        L.scg_table_key_words.argtypes = [C.c_void_p]
         L.scg_table_keys.restype = C.c_void_p
         L.scg_table_keys.argtypes = [C.c_void_p]
         L.scg_table_counts.restype = C.c_void_p
@@ -106,7 +107,7 @@ EXPORTS = [
     "scg_single_plan_create", "scg_single_plan_run", "scg_plan_free", "scg_plan_kernel",
     "scg_dual_plan_create", "scg_dual_plan_run", "scg_combo_plan_create", "scg_combo_plan_run",
     "scg_random_plan_create", "scg_random_plan_run", "scg_plan_reset", "scg_plan_harvest",
-    "scg_plan_sorted_table", "scg_plan_dense_tally", "scg_table_rows", "scg_table_key_len", "scg_table_keys", "scg_table_counts",
+    "scg_plan_sorted_table", "scg_plan_dense_tally", "scg_table_rows", "scg_table_key_len", "scg_table_key_words", "scg_table_keys", "scg_table_counts",
     "scg_table_from_device", "scg_table_merge", "scg_table_render", "scg_table_free",
     "scg_host_pack_roundtrip", "scg_jit_selftest", "scg_jit_selftest_uniform", "scg_jit_selftest_handler",
     "scg_device_alloc", "scg_device_free", "scg_device_zero", "scg_device_to_host", "scg_synchronize",

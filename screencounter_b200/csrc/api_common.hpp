@@ -13,6 +13,9 @@
 
 namespace scg {
 
+// 64-bit words per row of a sorted table's keys (SortedTable): two for random barcodes longer than 21 bases, one otherwise
+inline int table_key_words(int key_len) { return key_len > 21 ? 2 : 1; }
+
 std::string& creation_error();   // message of a failed scg_ctx_create
 
 // Runs f(); any exception becomes status 1 + ctx->last_error (BEGIN_RCPP/END_RCPP equivalent,
@@ -173,12 +176,19 @@ void launch_single(Context& ctx, const ReadsDev& reads, const SingleMatcher& m, 
                    uint32_t* d_info, cudaStream_t stream);
 
 // A sparse result resident on the device, sorted: what scg_result hands out on demand (scg_result_copy_table) and what the
-// multi-GPU merge exchanges.  keys: one 64-bit word per row, ascending -- combinations as first << 32 | second, random
-// barcodes as three bits per base in text order (A < C < G < N < T), first base most significant.
+// multi-GPU merge exchanges.  keys: table_key_words(key_len) 64-bit words per row, row-major, rows ascending by (word 0,
+// word 1):
+//   combinations            one word, first << 32 | second;
+//   random barcodes <= 21   one word, three bits per base in text order (A=0 < C=1 < G=2 < N=3 < T=4), first base most
+//                           significant;
+//   random barcodes 22..42  two words: word 0 = the ranks of bases 0..20 (the one-word key of the first 21 bases), word 1 =
+//                           the ranks of bases 21..key_len-1 in the same convention.
+// Every word is below 2^63, so int64 views keep the order.
 struct SortedTable {
-    DeviceBuffer keys, counts;   // unsigned long long[rows], uint32_t[rows]
+    DeviceBuffer keys, counts;   // unsigned long long[rows * words()], uint32_t[rows]
     size_t rows = 0;
     int key_len = 0;             // > 0: random barcodes of this length; 0: combinations
+    int words() const { return table_key_words(key_len); }
 };
 
 // Device count table (libdev.hpp: 16-byte slots for 64-bit keys, separate arrays for 128-bit keys).  Sized for a load
@@ -199,11 +209,8 @@ struct CountTable {
     void check_overflow(Context& ctx);                        // throws when inserts were dropped (synchronises)
     CountTable64 view64() const;
     CountTable128 view128() const;
-    // live entries to the host, unsorted (wide tables)
-    void download(Context& ctx, std::vector<unsigned long long>& keys_lo, std::vector<unsigned long long>& keys_hi,
-                  std::vector<uint32_t>& counts);
-    // narrow tables: live entries sorted on the device.  key_len > 0: keys are random barcodes (random_key64), re-coded to
-    // text order before the sort; key_len == 0: sorted as they are (combinations).
+    // live entries sorted on the device (SortedTable).  key_len > 0: keys are random barcodes (random_key64, or random_key128
+    // in a wide table), re-coded to text order before the sort; key_len == 0: sorted as they are (combinations).
     void sorted(Context& ctx, int key_len, SortedTable& out);
 };
 

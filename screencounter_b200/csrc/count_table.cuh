@@ -68,23 +68,37 @@ __device__ __forceinline__ ulonglong2 cas128(ulonglong2* addr, ulonglong2 expect
     return old;
 }
 
-__device__ __forceinline__ void count_insert128(const CountTable128& t, ulonglong2 key, uint32_t add) {
-    unsigned long long pos = count_hash(key.x ^ count_hash(key.y)) & t.mask;
+// Home of a 128-bit key: an EVEN slot, as count_home, so that the home and the slot after it are one aligned 32-byte sector
+// of keys.  Every kernel that inserts into a wide table starts at this home and probes slot by slot from it.
+__device__ __forceinline__ unsigned long long count_home128(const CountTable128& t, ulonglong2 key) {
+    return count_hash(key.x ^ count_hash(key.y)) & t.mask & ~1ull;
+}
+
+// Adds `add` to the count of `key`, inserting it when new.  Returns true when the key was new; the caller accounts for it
+// in t.live[0].
+__device__ __forceinline__ bool count_add128(const CountTable128& t, ulonglong2 key, uint32_t add) {
+    unsigned long long pos = count_home128(t, key);
     const ulonglong2 empty = make_ulonglong2(~0ull, ~0ull);
+    bool fresh = false;
     for (unsigned long long probes = 0;; ++probes) {
         const ulonglong2 old = cas128(t.keys + pos, empty, key);
         if (old.x == ~0ull && old.y == ~0ull) {
-            atomicAdd(t.live, 1ull);
+            fresh = true;
             break;
         }
         if (old.x == key.x && old.y == key.y) break;
         if (probes >= COUNT_MAX_PROBES || probes > t.mask) {
             atomicExch(t.live + 1, 1ull);
-            return;
+            return false;
         }
         pos = (pos + 1) & t.mask;
     }
     atomicAdd(t.counts + pos, add);
+    return fresh;
+}
+
+__device__ __forceinline__ void count_insert128(const CountTable128& t, ulonglong2 key, uint32_t add) {
+    if (count_add128(t, key, add)) atomicAdd(t.live, 1ull);
 }
 
 __device__ __forceinline__ void combo_count(const ComboSink& k, int id0, int id1) {
@@ -98,6 +112,12 @@ __device__ __forceinline__ void combo_count(const ComboSink& k, int id0, int id1
 // packed key of a random barcode of up to 21 bases: H | L << 21 | N << 42 (bit i of a plane = base i)
 __device__ __forceinline__ unsigned long long random_key64(uint32_t h, uint32_t l, uint32_t n) {
     return (unsigned long long)h | ((unsigned long long)l << 21) | ((unsigned long long)n << 42);
+}
+
+// packed key of a random barcode of 22 to 42 bases: the planes H, L, N (bit i = base i) in 42-bit fields of 128 bits,
+// x = H | L << 42, y = L >> 22 | N << 20 (y < 2^62, so no key is the empty slot's (~0, ~0))
+__device__ __forceinline__ ulonglong2 random_key128(unsigned long long h, unsigned long long l, unsigned long long n) {
+    return make_ulonglong2(h | (l << 42), (l >> 22) | (n << 20));
 }
 
 } // namespace scg

@@ -202,10 +202,7 @@ __global__ void __launch_bounds__(128) random_kernel(ReadsDev reads, RandomParam
                             L |= (unsigned long long)key.l[KW > 1 ? 1 : 0] << 32;
                             N |= (unsigned long long)key.n[KW > 1 ? 1 : 0] << 32;
                         }
-                        ulonglong2 k;
-                        k.x = H | (L << 42);
-                        k.y = (L >> 22) | (N << 20);
-                        count_insert128(t128, k, 1u);
+                        count_insert128(t128, random_key128(H, L, N), 1u);
                     }
                 }
             }

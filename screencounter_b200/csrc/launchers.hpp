@@ -26,7 +26,7 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
 long long count_single_core(Context& c, FastqReader* reader, const SingleMatcher& m, int nthreads, int32_t* d_counts, TraceSink& sink);
 
 // A sparse result (combinations, random barcodes) of one input or one part of it: a sorted table on the device, or -- random
-// barcodes taken from raw read text or longer than 21 bases -- a table rendered on the host.
+// barcodes taken from raw read text -- a table rendered on the host.
 struct SparseCounts {
     SortedTable table;
     std::unique_ptr<scg_result> rendered;   // set instead of `table`

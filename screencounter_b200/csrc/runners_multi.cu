@@ -179,9 +179,10 @@ void bring_home(Context& c0, SortedTable& t) {
     SortedTable here;
     here.rows = t.rows;
     here.key_len = t.key_len;
-    here.keys.alloc(t.rows * 8, false);
+    const size_t key_bytes = t.rows * 8 * (size_t)t.words();
+    here.keys.alloc(key_bytes, false);
     here.counts.alloc(t.rows * sizeof(uint32_t), false);
-    SCG_CUDA_CHECK(cudaMemcpyPeerAsync(here.keys.ptr, c0.device, t.keys.ptr, t.keys.device, t.rows * 8, c0.stream));
+    SCG_CUDA_CHECK(cudaMemcpyPeerAsync(here.keys.ptr, c0.device, t.keys.ptr, t.keys.device, key_bytes, c0.stream));
     SCG_CUDA_CHECK(cudaMemcpyPeerAsync(here.counts.ptr, c0.device, t.counts.ptr, t.counts.device, t.rows * sizeof(uint32_t), c0.stream));
     SCG_CUDA_CHECK(cudaStreamSynchronize(c0.stream));
     t = std::move(here);
@@ -200,8 +201,8 @@ void union_on_device(Context& c0, std::vector<SortedTable>& tables, SortedTable&
     if (tables.size() == 1) u = std::move(tables[0]);
 }
 
-// The union made on the host, for tables of which some could only be rendered there (random barcodes read from raw text, or
-// longer than 21 bases): key -> its count in every table.  std::map iterates strings in byte order = sort(union) of R for
+// The union made on the host, for tables of which some could only be rendered there (random barcodes read from raw text):
+// key -> its count in every table.  std::map iterates strings in byte order = sort(union) of R for
 // ACGTN text; combinations are keyed big-endian, so that byte order is (first, second) order.
 using HostUnion = std::map<std::string, std::vector<int32_t>>;
 HostUnion union_on_host(Context& c0, std::vector<SortedTable>& tables, std::vector<std::unique_ptr<scg_result>>& rendered, int width,

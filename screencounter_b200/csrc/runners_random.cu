@@ -49,16 +49,20 @@ __global__ void rehash128_kernel(const ulonglong2* keys, const uint32_t* counts,
 
 // Rank of every base in the byte order of its letter (A < C < G < N < T, what R's order() sees,
 // R/countRandomBarcodes.R:73), three bits per base, first base most significant: sorting these integers sorts the
-// barcodes as text.  Keys of up to 21 bases (random_key64: H | L << 21 | N << 42).
-__device__ __forceinline__ unsigned long long text_order_key(unsigned long long k, int len) {
-    const uint32_t H = (uint32_t)(k & 0x1FFFFFull), L = (uint32_t)((k >> 21) & 0x1FFFFFull), N = (uint32_t)((k >> 42) & 0x1FFFFFull);
+// barcodes as text.  Bases [from, to) of the planes H, L, N (bit b = base b).
+__device__ __forceinline__ unsigned long long text_order_bits(unsigned long long H, unsigned long long L, unsigned long long N, int from, int to) {
     unsigned long long s = 0;
-    for (int b = 0; b < len; ++b) {
-        const uint32_t code = (((H >> b) & 1u) << 1) | ((L >> b) & 1u);
-        const uint32_t rank = ((N >> b) & 1u) ? 3u : (code == 3u ? 4u : code);
+    for (int b = from; b < to; ++b) {
+        const uint32_t code = (uint32_t)((((H >> b) & 1ull) << 1) | ((L >> b) & 1ull));
+        const uint32_t rank = ((N >> b) & 1ull) ? 3u : (code == 3u ? 4u : code);
         s = (s << 3) | rank;
     }
     return s;
+}
+
+// Keys of up to 21 bases (random_key64: H | L << 21 | N << 42).
+__device__ __forceinline__ unsigned long long text_order_key(unsigned long long k, int len) {
+    return text_order_bits(k & 0x1FFFFFull, (k >> 21) & 0x1FFFFFull, (k >> 42) & 0x1FFFFFull, 0, len);
 }
 
 // compact the live entries of a narrow table (key_len > 0: keys re-coded to text order on the way); one atomic per warp
@@ -86,15 +90,47 @@ __global__ void compact64_kernel(const CountSlot* slots, size_t n, int key_len, 
     }
 }
 
-__global__ void compact128_kernel(const ulonglong2* keys, const uint32_t* counts, size_t n,
-                                  ulonglong2* out_keys, uint32_t* out_counts, unsigned long long* cursor) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        if (!(keys[i].x == ~0ull && keys[i].y == ~0ull)) {
-            const unsigned long long at = atomicAdd(cursor, 1ull);
-            out_keys[at] = keys[i];
+// A row of a wide sorted table (SortedTable: two text-order words), and how the radix sort sees it: word 0 most significant.
+struct WideKey {
+    unsigned long long w0, w1;
+};
+__device__ __forceinline__ bool operator<(const WideKey& a, const WideKey& b) { return a.w0 < b.w0 || (a.w0 == b.w0 && a.w1 < b.w1); }
+__device__ __forceinline__ bool operator==(const WideKey& a, const WideKey& b) { return a.w0 == b.w0 && a.w1 == b.w1; }
+struct WideKeyDecomposer {
+    __host__ __device__ ::cuda::std::tuple<unsigned long long&, unsigned long long&> operator()(WideKey& k) const { return { k.w0, k.w1 }; }
+};
+
+// compact the live entries of a wide table, one atomic per warp, keys re-coded on the way to the two text-order words, word 1
+// shifted up by `shift1` bits: the 3 * key_len bits in use are then the contiguous bits [shift1, 127) of (word 0, word 1),
+// the only ones the radix sort has to look at
+__global__ void compact128_kernel(const ulonglong2* keys, const uint32_t* counts, size_t n, int key_len, int shift1, WideKey* out_keys,
+                                  uint32_t* out_counts, unsigned long long* cursor) {
+    const int lane = threadIdx.x & 31;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    const size_t rounds = (n + stride - 1) / stride;
+    const unsigned long long m42 = (1ull << 42) - 1;
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    for (size_t r = 0; r < rounds; ++r, i += stride) {
+        ulonglong2 k = make_ulonglong2(~0ull, ~0ull);
+        if (i < n) k = keys[i];
+        const bool livep = !(k.x == ~0ull && k.y == ~0ull);
+        const uint32_t m = __ballot_sync(0xFFFFFFFFu, livep);
+        if (!m) continue;
+        unsigned long long base = 0;
+        const int leader = __ffs(m) - 1;
+        if (lane == leader) base = atomicAdd(cursor, (unsigned long long)__popc(m));
+        base = __shfl_sync(0xFFFFFFFFu, base, leader);
+        if (livep) {
+            const unsigned long long at = base + __popc(m & ((1u << lane) - 1u));
+            const unsigned long long H = k.x & m42, L = ((k.x >> 42) | (k.y << 22)) & m42, N = (k.y >> 20) & m42;
+            out_keys[at] = WideKey{ text_order_bits(H, L, N, 0, 21), text_order_bits(H, L, N, 21, key_len) << shift1 };
             out_counts[at] = counts[i];
         }
     }
+}
+
+__global__ void unshift_word1_kernel(WideKey* keys, size_t n, int shift1) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) keys[i].w1 >>= shift1;
 }
 
 static int fill_grid(Context& ctx, size_t n) { return (int)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)ctx.sm_count * 32)); }
@@ -190,83 +226,71 @@ void CountTable::ensure(Context& ctx, long long upcoming) {
     pending += upcoming;
 }
 
-void CountTable::download(Context& ctx, std::vector<unsigned long long>& keys_lo, std::vector<unsigned long long>& keys_hi,
-                          std::vector<uint32_t>& out_counts) {
-    check_overflow(ctx);
-    const size_t nlive = (size_t)live_known;
-    keys_lo.resize(nlive);
-    keys_hi.clear();
-    out_counts.resize(nlive);
-    if (nlive == 0) return;
-    DeviceBuffer d_keys, d_counts, d_cursor;
-    d_keys.alloc(nlive * 16, false);
-    d_counts.alloc(nlive * sizeof(uint32_t), false);
-    d_cursor.alloc(sizeof(unsigned long long), true);
-    if (wide) {
-        compact128_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<ulonglong2>(), counts.as<uint32_t>(), capacity,
-                                                                          d_keys.as<ulonglong2>(), d_counts.as<uint32_t>(),
-                                                                          d_cursor.as<unsigned long long>());
-    } else {
-        compact64_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<CountSlot>(), capacity, 0, d_keys.as<unsigned long long>(),
-                                                                         d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
-    }
-    SCG_CUDA_CHECK(cudaGetLastError());
-    ++ctx.launches;
-    SCG_CUDA_CHECK(cudaMemcpyAsync(out_counts.data(), d_counts.ptr, nlive * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx.stream));
-    if (wide) {
-        std::vector<ulonglong2> tmp(nlive);
-        SCG_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), d_keys.ptr, nlive * 16, cudaMemcpyDeviceToHost, ctx.stream));
-        SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-        keys_hi.resize(nlive);
-        for (size_t i = 0; i < nlive; ++i) {
-            keys_lo[i] = tmp[i].x;
-            keys_hi[i] = tmp[i].y;
-        }
-    } else {
-        SCG_CUDA_CHECK(cudaMemcpyAsync(keys_lo.data(), d_keys.ptr, nlive * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-    }
-}
-
-// Live entries of a narrow table as (key, count) sorted by key ON THE DEVICE (radix sort), left there.
+// Live entries as (key, count) sorted by key ON THE DEVICE (radix sort), left there in the layout of SortedTable.
 void CountTable::sorted(Context& ctx, int key_len, SortedTable& out) {
-    if (wide) throw Error("internal error: only narrow count tables are sorted on the device");
+    if (wide != (table_key_words(key_len) == 2)) throw Error("internal error: count table and key length disagree on the key width");
     check_overflow(ctx);
     const size_t nlive = (size_t)live_known;
     out.rows = nlive;
     out.key_len = key_len;
-    out.keys.alloc(std::max<size_t>(nlive, 1) * 8, false);
+    const size_t key_bytes = 8 * (size_t)out.words();
+    out.keys.alloc(std::max<size_t>(nlive, 1) * key_bytes, false);
     out.counts.alloc(std::max<size_t>(nlive, 1) * sizeof(uint32_t), false);
     if (nlive == 0) return;
     DeviceBuffer d_keys, d_counts, d_cursor, d_temp;
-    d_keys.alloc(nlive * 8, false);
+    d_keys.alloc(nlive * key_bytes, false);
     d_counts.alloc(nlive * sizeof(uint32_t), false);
     d_cursor.alloc(sizeof(unsigned long long), true);
-    compact64_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<CountSlot>(), capacity, key_len, d_keys.as<unsigned long long>(),
-                                                                     d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
-    SCG_CUDA_CHECK(cudaGetLastError());
-    const int end_bit = key_len > 0 ? 3 * key_len : 64;
     size_t temp_bytes = 0;
-    SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_keys.as<unsigned long long>(), out.keys.as<unsigned long long>(),
-                                                   d_counts.as<uint32_t>(), out.counts.as<uint32_t>(), (long long)nlive, 0, end_bit, ctx.stream));
-    d_temp.alloc(temp_bytes, false);
-    SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(d_temp.ptr, temp_bytes, d_keys.as<unsigned long long>(), out.keys.as<unsigned long long>(),
-                                                   d_counts.as<uint32_t>(), out.counts.as<uint32_t>(), (long long)nlive, 0, end_bit, ctx.stream));
-    ctx.launches += 3;
+    if (wide) {
+        const int shift1 = 64 - 3 * (key_len - 21);
+        compact128_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<ulonglong2>(), counts.as<uint32_t>(), capacity, key_len, shift1,
+                                                                          d_keys.as<WideKey>(), d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
+        SCG_CUDA_CHECK(cudaGetLastError());
+        SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_keys.as<WideKey>(), out.keys.as<WideKey>(), d_counts.as<uint32_t>(),
+                                                       out.counts.as<uint32_t>(), (long long)nlive, WideKeyDecomposer{}, shift1, 127, ctx.stream));
+        d_temp.alloc(temp_bytes, false);
+        SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(d_temp.ptr, temp_bytes, d_keys.as<WideKey>(), out.keys.as<WideKey>(), d_counts.as<uint32_t>(),
+                                                       out.counts.as<uint32_t>(), (long long)nlive, WideKeyDecomposer{}, shift1, 127, ctx.stream));
+        unshift_word1_kernel<<<fill_grid(ctx, nlive), 256, 0, ctx.stream>>>(out.keys.as<WideKey>(), nlive, shift1);
+        SCG_CUDA_CHECK(cudaGetLastError());
+        ctx.launches += 4;
+    } else {
+        compact64_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<CountSlot>(), capacity, key_len, d_keys.as<unsigned long long>(),
+                                                                         d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
+        SCG_CUDA_CHECK(cudaGetLastError());
+        const int end_bit = key_len > 0 ? 3 * key_len : 64;
+        SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_keys.as<unsigned long long>(), out.keys.as<unsigned long long>(),
+                                                       d_counts.as<uint32_t>(), out.counts.as<uint32_t>(), (long long)nlive, 0, end_bit, ctx.stream));
+        d_temp.alloc(temp_bytes, false);
+        SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(d_temp.ptr, temp_bytes, d_keys.as<unsigned long long>(), out.keys.as<unsigned long long>(),
+                                                       d_counts.as<uint32_t>(), out.counts.as<uint32_t>(), (long long)nlive, 0, end_bit, ctx.stream));
+        ctx.launches += 3;
+    }
     SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));   // the scratch buffers above go back to the block cache
 }
 
 // ---------------------------------------------------------------------------------------
 // sorted tables: rendering and merging on the device
 // ---------------------------------------------------------------------------------------
+// one row per thread; a wide key (words == 2) renders bases 0..20 from word 0 and the rest from word 1
 __global__ void render_barcodes_kernel(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ counts, size_t n, int len,
-                                       char* __restrict__ strings, int32_t* __restrict__ freq) {
+                                       int words, char* __restrict__ strings, int32_t* __restrict__ freq) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        unsigned long long k = keys[i];
+        const unsigned long long* row = keys + i * (size_t)words;
         char* out = strings + i * (size_t)len;
-        for (int b = len - 1; b >= 0; --b) {
+        const int len0 = words == 2 ? 21 : len;
+        unsigned long long k = row[0];
+        for (int b = len0 - 1; b >= 0; --b) {
             out[b] = "ACGNT"[k & 7ull];
             k >>= 3;
+        }
+        if (words == 2) {
+            k = row[1];
+            for (int b = len - 1; b >= 21; --b) {
+                out[b] = "ACGNT"[k & 7ull];
+                k >>= 3;
+            }
         }
         freq[i] = (int32_t)counts[i];
     }
@@ -277,7 +301,7 @@ void render_barcodes(Context& ctx, const SortedTable& t, DeviceBuffer& strings, 
     freq.alloc(std::max<size_t>(t.rows, 4) * sizeof(int32_t), false);
     if (t.rows == 0) return;
     render_barcodes_kernel<<<fill_grid(ctx, t.rows), 256, 0, ctx.stream>>>(t.keys.as<unsigned long long>(), t.counts.as<uint32_t>(), t.rows, t.key_len,
-                                                                          strings.as<char>(), freq.as<int32_t>());
+                                                                          t.words(), strings.as<char>(), freq.as<int32_t>());
     SCG_CUDA_CHECK(cudaGetLastError());
     ++ctx.launches;
 }
@@ -319,8 +343,10 @@ void device_table_result(Context& ctx, const SortedTable& t, scg_result& out) {
 // Merge of two sorted tables (the device-side reduce() of handlers/RandomBarcodeSingleEnd.hpp:197-207 and of the
 // combinations' append + sort, handlers/CombinatorialBarcodesSingleEnd.hpp:268-305): every row finds its place in the
 // output by a binary search in the OTHER table -- rank = own index + rows of the other table that sort before it, minus
-// the keys both tables hold that sort before it (those collapse into one row).
-__device__ __forceinline__ size_t lower_bound_dev(const unsigned long long* __restrict__ a, size_t n, unsigned long long key) {
+// the keys both tables hold that sort before it (those collapse into one row).  K: the row's key, one word
+// (unsigned long long) or two (WideKey).
+template <class K>
+__device__ __forceinline__ size_t lower_bound_dev(const K* __restrict__ a, size_t n, K key) {
     size_t lo = 0, hi = n;
     while (lo < hi) {
         const size_t mid = (lo + hi) >> 1;
@@ -334,40 +360,54 @@ __device__ __forceinline__ size_t lower_bound_dev(const unsigned long long* __re
 }
 
 // pass 1: for every row of a, 1 if b also holds its key (those rows of b are dropped)
-__global__ void merge_mark_kernel(const unsigned long long* __restrict__ ak, size_t na, const unsigned long long* __restrict__ bk, size_t nb,
-                                  uint32_t* __restrict__ a_pos_in_b, uint32_t* __restrict__ b_dup) {
+template <class K>
+__global__ void merge_mark_kernel(const K* __restrict__ ak, size_t na, const K* __restrict__ bk, size_t nb, uint32_t* __restrict__ a_pos_in_b,
+                                  uint32_t* __restrict__ b_dup) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < na; i += (size_t)gridDim.x * blockDim.x) {
-        const size_t p = lower_bound_dev(bk, nb, ak[i]);
+        const K key = ak[i];
+        const size_t p = lower_bound_dev(bk, nb, key);
         a_pos_in_b[i] = (uint32_t)p;
-        if (p < nb && bk[p] == ak[i]) b_dup[p] = 1;
+        if (p < nb && bk[p] == key) b_dup[p] = 1;
     }
 }
 
 // pass 2 (after an exclusive scan of b_dup): scatter
-__global__ void merge_scatter_a_kernel(const unsigned long long* __restrict__ ak, const uint32_t* __restrict__ ac, size_t na,
-                                       const unsigned long long* __restrict__ bk, const uint32_t* __restrict__ bc, size_t nb,
-                                       const uint32_t* __restrict__ a_pos_in_b, const uint32_t* __restrict__ dup_before,
-                                       unsigned long long* __restrict__ ck, uint32_t* __restrict__ cc) {
+template <class K>
+__global__ void merge_scatter_a_kernel(const K* __restrict__ ak, const uint32_t* __restrict__ ac, size_t na, const K* __restrict__ bk,
+                                       const uint32_t* __restrict__ bc, size_t nb, const uint32_t* __restrict__ a_pos_in_b,
+                                       const uint32_t* __restrict__ dup_before, K* __restrict__ ck, uint32_t* __restrict__ cc) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < na; i += (size_t)gridDim.x * blockDim.x) {
         const size_t p = a_pos_in_b[i];
         // rows of b before p that survive = p - duplicates among them
         const size_t at = i + p - dup_before[p];
+        const K key = ak[i];
         uint32_t count = ac[i];
-        if (p < nb && bk[p] == ak[i]) count += bc[p];
-        ck[at] = ak[i];
+        if (p < nb && bk[p] == key) count += bc[p];
+        ck[at] = key;
         cc[at] = count;
     }
 }
 
-__global__ void merge_scatter_b_kernel(const unsigned long long* __restrict__ ak, size_t na, const unsigned long long* __restrict__ bk,
-                                       const uint32_t* __restrict__ bc, size_t nb, const uint32_t* __restrict__ b_dup,
-                                       const uint32_t* __restrict__ dup_before, unsigned long long* __restrict__ ck, uint32_t* __restrict__ cc) {
+template <class K>
+__global__ void merge_scatter_b_kernel(const K* __restrict__ ak, size_t na, const K* __restrict__ bk, const uint32_t* __restrict__ bc, size_t nb,
+                                       const uint32_t* __restrict__ b_dup, const uint32_t* __restrict__ dup_before, K* __restrict__ ck,
+                                       uint32_t* __restrict__ cc) {
     for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < nb; j += (size_t)gridDim.x * blockDim.x) {
         if (b_dup[j]) continue;
         const size_t q = lower_bound_dev(ak, na, bk[j]);   // rows of a before it (its key is not in a)
         const size_t at = q + j - dup_before[j];
         ck[at] = bk[j];
         cc[at] = bc[j];
+    }
+}
+
+// f(K{}) with the key type of tables of `words` words per row
+template <class F>
+static void with_key_type(int words, F&& f) {
+    if (words == 2) {
+        f(WideKey{});
+    } else {
+        f(0ull);
     }
 }
 
@@ -380,49 +420,56 @@ void merge_sorted_tables(Context& ctx, const SortedTable& a, const SortedTable& 
     dup.alloc((nb + 1) * sizeof(uint32_t), false);
     dup_scan.alloc((nb + 1) * sizeof(uint32_t), false);
     SCG_CUDA_CHECK(cudaMemsetAsync(dup.ptr, 0, (nb + 1) * sizeof(uint32_t), ctx.stream));
-    if (na) {
-        merge_mark_kernel<<<fill_grid(ctx, na), 256, 0, ctx.stream>>>(a.keys.as<unsigned long long>(), na, b.keys.as<unsigned long long>(), nb,
-                                                                     pos.as<uint32_t>(), dup.as<uint32_t>());
-        SCG_CUDA_CHECK(cudaGetLastError());
-    }
-    size_t temp_bytes = 0;
-    SCG_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, dup.as<uint32_t>(), dup_scan.as<uint32_t>(), (long long)(nb + 1), ctx.stream));
-    d_temp.alloc(temp_bytes, false);
-    SCG_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(d_temp.ptr, temp_bytes, dup.as<uint32_t>(), dup_scan.as<uint32_t>(), (long long)(nb + 1), ctx.stream));
-    uint32_t ndup = 0;
-    SCG_CUDA_CHECK(cudaMemcpyAsync(&ndup, dup_scan.as<uint32_t>() + nb, sizeof ndup, cudaMemcpyDeviceToHost, ctx.stream));
-    SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-    c.rows = na + nb - ndup;
-    c.keys.alloc(std::max<size_t>(c.rows, 1) * 8, false);
-    c.counts.alloc(std::max<size_t>(c.rows, 1) * sizeof(uint32_t), false);
-    if (na) {
-        merge_scatter_a_kernel<<<fill_grid(ctx, na), 256, 0, ctx.stream>>>(a.keys.as<unsigned long long>(), a.counts.as<uint32_t>(), na,
-                                                                          b.keys.as<unsigned long long>(), b.counts.as<uint32_t>(), nb, pos.as<uint32_t>(),
-                                                                          dup_scan.as<uint32_t>(), c.keys.as<unsigned long long>(), c.counts.as<uint32_t>());
-    }
-    if (nb) {
-        merge_scatter_b_kernel<<<fill_grid(ctx, nb), 256, 0, ctx.stream>>>(a.keys.as<unsigned long long>(), na, b.keys.as<unsigned long long>(),
-                                                                          b.counts.as<uint32_t>(), nb, dup.as<uint32_t>(), dup_scan.as<uint32_t>(),
-                                                                          c.keys.as<unsigned long long>(), c.counts.as<uint32_t>());
-    }
+    with_key_type(c.words(), [&](auto key) {
+        using K = decltype(key);
+        if (na) {
+            merge_mark_kernel<K><<<fill_grid(ctx, na), 256, 0, ctx.stream>>>(a.keys.as<K>(), na, b.keys.as<K>(), nb, pos.as<uint32_t>(), dup.as<uint32_t>());
+            SCG_CUDA_CHECK(cudaGetLastError());
+        }
+        size_t temp_bytes = 0;
+        SCG_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, dup.as<uint32_t>(), dup_scan.as<uint32_t>(), (long long)(nb + 1), ctx.stream));
+        d_temp.alloc(temp_bytes, false);
+        SCG_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(d_temp.ptr, temp_bytes, dup.as<uint32_t>(), dup_scan.as<uint32_t>(), (long long)(nb + 1), ctx.stream));
+        uint32_t ndup = 0;
+        SCG_CUDA_CHECK(cudaMemcpyAsync(&ndup, dup_scan.as<uint32_t>() + nb, sizeof ndup, cudaMemcpyDeviceToHost, ctx.stream));
+        SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        c.rows = na + nb - ndup;
+        c.keys.alloc(std::max<size_t>(c.rows, 1) * sizeof(K), false);
+        c.counts.alloc(std::max<size_t>(c.rows, 1) * sizeof(uint32_t), false);
+        if (na) {
+            merge_scatter_a_kernel<K><<<fill_grid(ctx, na), 256, 0, ctx.stream>>>(a.keys.as<K>(), a.counts.as<uint32_t>(), na, b.keys.as<K>(),
+                                                                                b.counts.as<uint32_t>(), nb, pos.as<uint32_t>(), dup_scan.as<uint32_t>(),
+                                                                                c.keys.as<K>(), c.counts.as<uint32_t>());
+        }
+        if (nb) {
+            merge_scatter_b_kernel<K><<<fill_grid(ctx, nb), 256, 0, ctx.stream>>>(a.keys.as<K>(), na, b.keys.as<K>(), b.counts.as<uint32_t>(), nb,
+                                                                                dup.as<uint32_t>(), dup_scan.as<uint32_t>(), c.keys.as<K>(),
+                                                                                c.counts.as<uint32_t>());
+        }
+    });
     SCG_CUDA_CHECK(cudaGetLastError());
     ctx.launches += 5;
     SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
 }
 
 // column[i] = count of all_keys[i] in table t, 0 where t does not hold the key (every key of t is in all_keys)
-__global__ void scatter_column_kernel(const unsigned long long* __restrict__ uk, size_t nu, const unsigned long long* __restrict__ tk,
-                                      const uint32_t* __restrict__ tc, size_t nt, int32_t* __restrict__ column) {
+template <class K>
+__global__ void scatter_column_kernel(const K* __restrict__ uk, size_t nu, const K* __restrict__ tk, const uint32_t* __restrict__ tc, size_t nt,
+                                      int32_t* __restrict__ column) {
     for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < nt; j += (size_t)gridDim.x * blockDim.x) {
-        const size_t p = lower_bound_dev(uk, nu, tk[j]);
-        if (p < nu && uk[p] == tk[j]) column[p] = (int32_t)tc[j];
+        const K key = tk[j];
+        const size_t p = lower_bound_dev(uk, nu, key);
+        if (p < nu && uk[p] == key) column[p] = (int32_t)tc[j];
     }
 }
 
 void scatter_table_column(Context& ctx, const SortedTable& all_keys, const SortedTable& t, int32_t* column) {
     if (t.rows == 0) return;
-    scatter_column_kernel<<<fill_grid(ctx, t.rows), 256, 0, ctx.stream>>>(all_keys.keys.as<unsigned long long>(), all_keys.rows,
-                                                                         t.keys.as<unsigned long long>(), t.counts.as<uint32_t>(), t.rows, column);
+    with_key_type(t.words(), [&](auto key) {
+        using K = decltype(key);
+        scatter_column_kernel<K><<<fill_grid(ctx, t.rows), 256, 0, ctx.stream>>>(all_keys.keys.as<K>(), all_keys.rows, t.keys.as<K>(),
+                                                                                t.counts.as<uint32_t>(), t.rows, column);
+    });
     SCG_CUDA_CHECK(cudaGetLastError());
     ++ctx.launches;
 }
@@ -543,34 +590,6 @@ void ComboTally::harvest(Context& ctx, scg_result& out) {
     device_table_result(ctx, t, out);
 }
 
-namespace {
-
-// Decodes a packed random-barcode key (random_kernel's layout) to text.
-std::string decode_key(unsigned long long lo, unsigned long long hi, int len, bool wide) {
-    unsigned long long H, L, N;
-    if (!wide) {
-        H = lo & ((1ull << 21) - 1);
-        L = (lo >> 21) & ((1ull << 21) - 1);
-        N = (lo >> 42) & ((1ull << 21) - 1);
-    } else {
-        const unsigned long long m42 = (1ull << 42) - 1;
-        H = lo & m42;
-        L = ((lo >> 42) | (hi << 22)) & m42;
-        N = (hi >> 20) & m42;
-    }
-    std::string s(len, 'A');
-    for (int i = 0; i < len; ++i) {
-        if ((N >> i) & 1ull) {
-            s[i] = 'N';
-        } else {
-            s[i] = "ACGT"[(((H >> i) & 1ull) << 1) | ((L >> i) & 1ull)];
-        }
-    }
-    return s;
-}
-
-} // namespace
-
 } // namespace scg
 
 using namespace scg;
@@ -581,8 +600,8 @@ extern "C" {
 
 namespace scg {
 
-// countRandomBarcodes over one reader.  Barcodes of up to 21 bases, none taken from raw read text, stay on the device as a
-// sorted table (rank-coded, text order); any other result is rendered on the host.
+// countRandomBarcodes over one reader.  The barcodes stay on the device as a sorted table (rank-coded, text order); only when
+// some were taken from raw read text is the result rendered on the host.
 void count_random_reader(Context& c, FastqReader* reader, const RandomMatcher& m, int nthreads, SparseCounts& result) {
     const TemplateSpec& tmpl = m.tmpl;
     const int key_len = m.key_len;
@@ -654,69 +673,62 @@ void count_random_reader(Context& c, FastqReader* reader, const RandomMatcher& m
     }
     const double t_harvest = now_s();
     result.reads = nreads;
+    // sorted as text ON THE DEVICE (radix sort of rank-coded keys)
+    SortedTable sorted;
+    tab.sorted(c, key_len, sorted);
+    if (extra.empty()) {
+        result.table = std::move(sorted);
+        c.timing.harvest_s = now_s() - t_harvest;
+        return;
+    }
+    // a few keys came from raw read text (lower case, IUPAC letters): merged on the host in text order
+    const size_t n = sorted.rows;
+    const int words = sorted.words();
+    std::vector<unsigned long long> order_keys(n * (size_t)words);
+    std::vector<uint32_t> cnt(n);
+    if (n) {
+        SCG_CUDA_CHECK(cudaMemcpyAsync(order_keys.data(), sorted.keys.ptr, order_keys.size() * 8, cudaMemcpyDeviceToHost, c.stream));
+        SCG_CUDA_CHECK(cudaMemcpyAsync(cnt.data(), sorted.counts.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+        SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
+    }
+    // one row of the table as text: bases 0..20 (or all of a narrow key) from word 0, the rest from word 1
+    auto render = [&](const unsigned long long* row, char* out) {
+        const int len0 = words == 2 ? 21 : key_len;
+        unsigned long long k = row[0];
+        for (int b = len0 - 1; b >= 0; --b) {
+            out[b] = "ACGNT"[k & 7ull];
+            k >>= 3;
+        }
+        k = words == 2 ? row[1] : 0ull;
+        for (int b = key_len - 1; b >= len0; --b) {
+            out[b] = "ACGNT"[k & 7ull];
+            k >>= 3;
+        }
+    };
     std::unique_ptr<scg_result> r(new scg_result);
     r->width = key_len;
-    if (!wide) {
-        // barcodes of up to 21 bases: sorted as text ON THE DEVICE (radix sort of rank-coded keys)
-        SortedTable sorted;
-        tab.sorted(c, key_len, sorted);
-        if (extra.empty()) {
-            result.table = std::move(sorted);
-            c.timing.harvest_s = now_s() - t_harvest;
-            return;
+    r->strings.reserve((n + extra.size()) * (size_t)key_len);
+    r->freq.reserve(n + extra.size());
+    std::string cur(key_len, ' ');
+    auto it = extra.begin();
+    auto emit = [&](const std::string& k, int f) {
+        r->strings.insert(r->strings.end(), k.begin(), k.end());
+        r->freq.push_back(f);
+    };
+    for (size_t i = 0; i < n; ++i) {
+        render(&order_keys[i * (size_t)words], &cur[0]);
+        while (it != extra.end() && it->first < cur) {
+            emit(it->first, it->second);
+            ++it;
         }
-        {
-            // a few keys came from raw read text (lower case, IUPAC letters): merged on the host in text order
-            const size_t n = sorted.rows;
-            std::vector<unsigned long long> order_keys(n);
-            std::vector<uint32_t> cnt(n);
-            if (n) {
-                SCG_CUDA_CHECK(cudaMemcpyAsync(order_keys.data(), sorted.keys.ptr, n * 8, cudaMemcpyDeviceToHost, c.stream));
-                SCG_CUDA_CHECK(cudaMemcpyAsync(cnt.data(), sorted.counts.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
-                SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
-            }
-            auto render = [&](unsigned long long k, char* out) {
-                for (int b = key_len - 1; b >= 0; --b) {
-                    out[b] = "ACGNT"[k & 7ull];
-                    k >>= 3;
-                }
-            };
-            r->strings.reserve((n + extra.size()) * (size_t)key_len);
-            r->freq.reserve(n + extra.size());
-            std::string cur(key_len, ' ');
-            auto it = extra.begin();
-            auto emit = [&](const std::string& k, int f) {
-                r->strings.insert(r->strings.end(), k.begin(), k.end());
-                r->freq.push_back(f);
-            };
-            for (size_t i = 0; i < n; ++i) {
-                render(order_keys[i], &cur[0]);
-                while (it != extra.end() && it->first < cur) {
-                    emit(it->first, it->second);
-                    ++it;
-                }
-                int f = (int)cnt[i];
-                if (it != extra.end() && it->first == cur) {
-                    f += it->second;
-                    ++it;
-                }
-                emit(cur, f);
-            }
-            for (; it != extra.end(); ++it) emit(it->first, it->second);
+        int f = (int)cnt[i];
+        if (it != extra.end() && it->first == cur) {
+            f += it->second;
+            ++it;
         }
-    } else {
-        std::vector<unsigned long long> lo, hi;
-        std::vector<uint32_t> cnt;
-        tab.download(c, lo, hi, cnt);
-        std::map<std::string, int> merged(std::move(extra));
-        for (size_t i = 0; i < lo.size(); ++i) merged[decode_key(lo[i], hi[i], key_len, wide)] += (int)cnt[i];
-        r->strings.reserve(merged.size() * (size_t)key_len);
-        r->freq.reserve(merged.size());
-        for (const auto& kv : merged) {  // std::map iterates in byte order = R's order(sequences) for ACGTN text
-            r->strings.insert(r->strings.end(), kv.first.begin(), kv.first.end());
-            r->freq.push_back(kv.second);
-        }
+        emit(cur, f);
     }
+    for (; it != extra.end(); ++it) emit(it->first, it->second);
     c.timing.harvest_s = now_s() - t_harvest;
     result.rendered = std::move(r);
 }

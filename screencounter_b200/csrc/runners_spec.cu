@@ -418,6 +418,29 @@ __global__ void __launch_bounds__(256) random_insert_kernel(DeferredList def, Co
     if (lane == 0 && fresh) atomicAdd(table.live, fresh);
 }
 
+// The same for a wide table (barcodes of 22 to 42 bases): an entry is the 128-bit key in four words, inserted (or found) by
+// the full probing loop from its even home (count_add128), the loop the generic kernel's inserts take.
+__global__ void __launch_bounds__(256) random_insert128_kernel(DeferredList def, CountTable128 table) {
+    const int lane = threadIdx.x & 31;
+    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint32_t nwarps = (gridDim.x * blockDim.x) >> 5;
+    unsigned long long fresh = 0;
+    for (uint32_t r = warp; r < def.regions; r += nwarps) {
+        const uint32_t cnt = def.warp_counts[r];
+        const unsigned long long base = (unsigned long long)r * def.per_warp;
+        for (uint32_t e = lane; e < cnt; e += 32) {
+            const unsigned long long at = base + e;
+            const ulonglong2 key = make_ulonglong2((unsigned long long)def.words[at] | ((unsigned long long)def.words[def.stride + at] << 32),
+                                                   (unsigned long long)def.words[2 * def.stride + at] |
+                                                       ((unsigned long long)def.words[3 * def.stride + at] << 32));
+            if (count_add128(table, key, 1u)) ++fresh;
+        }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) fresh += __shfl_xor_sync(0xFFFFFFFFu, fresh, d);
+    if (lane == 0 && fresh) atomicAdd(table.live, fresh);
+}
+
 // countRandomBarcodes, partitioned (libdev.hpp PartitionedKeys): the lists of table part 0 are counted first, then part 1's, ...
 // -- regions are numbered part-major and the warps take them in that order, so at any moment the kernel works on one or two
 // parts of the table, which stay in L2: the random traffic of the inserts never reaches HBM.  Four keys per lane in flight.
@@ -781,10 +804,6 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
     int nparts = 0;
     bool ok = !spec_disabled();
     if (!ok) why = "disabled by SCG_NO_SPEC_HANDLERS";
-    if (ok && m.wide) {
-        ok = false;
-        why = "barcodes longer than 21 bases use the generic kernel";
-    }
     if (ok) ok = template_fits(m.tmpl, m.params.spec, reads, &why);
     if (ok) {
         group = jit_env_int("SCG_SPH_GROUP", 2, 1, 8);
@@ -801,7 +820,7 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
             while (nparts && nparts < std::min(want, 32)) nparts *= 2;
         }
         while (nparts > 0 && (size_t)nparts * 2 > tab.capacity) nparts /= 2;
-        if (nparts < 2) nparts = 0;
+        if (nparts < 2 || m.wide) nparts = 0;   // a wide table takes the home-sector route at every size
         mod = jit_module(random_program(m.tmpl, m.params.spec, m.params.max_mm, reads, m.params.use_first, out_index ? 1 : 0, nparts ? 1 : 0),
                          ctx.device, &why);
     }
@@ -813,10 +832,11 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
     cudaKernel_t k = mod->kernels[0];
     const int grid = spec_grid(ctx, k, reads.n, group);
     // (the partitioned route keeps its key lists where the other route keeps its deferred entries: two words per read at most)
-    Scratch sc = prepare_scratch(ctx, reads.n, grid, group, nparts ? 0 : 2, stream);
+    Scratch sc = prepare_scratch(ctx, reads.n, grid, group, nparts ? 0 : (m.wide ? 4 : 2), stream);
     SlowList slow = sc.slow;
     ReadsDev a = reads;
     CountTable64 t64 = tab.view64();
+    CountTable128 t128 = tab.view128();
     long long read_offset = 0;
     PartitionedKeys parts{ nullptr, nullptr, 0, 0, 0, 0 };
     if (nparts) {
@@ -836,7 +856,8 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
         parts.counts = ctx.part_counts.as<uint32_t>();
         SCG_CUDA_CHECK(cudaMemsetAsync(parts.counts, 0, (size_t)parts.nparts * parts.nwarps * sizeof(uint32_t), stream));
     }
-    void* args[] = { &a, &t64, &odd, &read_offset, &odd_out, &odd_count, &out_index, &sc.def, &slow, &parts };
+    void* table_arg = m.wide ? static_cast<void*>(&t128) : static_cast<void*>(&t64);
+    void* args[] = { &a, table_arg, &odd, &read_offset, &odd_out, &odd_count, &out_index, &sc.def, &slow, &parts };
     SCG_CUDA_CHECK(cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3(grid), dim3(128), args, 0, stream));
     if (nparts) {
         // exactly the blocks that are resident together: every warp then walks the parts in the same order at the same pace, and
@@ -855,6 +876,8 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
         } else {
             launch(random_count_parts_kernel<4>);
         }
+    } else if (m.wide) {
+        random_insert128_kernel<<<ctx.sm_count * 8, 256, 0, stream>>>(sc.def, t128);
     } else {
         // barcodes that were not in their home sector yet: inserted (or found further along) by the follow-up kernel
         random_insert_kernel<<<ctx.sm_count * 8, 256, 0, stream>>>(sc.def, t64);
@@ -868,6 +891,8 @@ void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, 
     }
     ctx.kernel_note = nparts ? "specialised (NVRTC) spec_random_kernel, filter+verify, barcodes listed by table part (" + std::to_string(nparts) + " parts), " +
                                    std::to_string(specialised_blocks_per_sm(k)) + " blocks/SM; + random_count_parts_kernel (16-byte-slot count table filled part by part in L2)"
+                  : m.wide ? "specialised (NVRTC) spec_random_kernel, filter+verify + 128-bit-key count table (home sector requested a tile ahead), " +
+                                   std::to_string(specialised_blocks_per_sm(k)) + " blocks/SM; + random_insert128_kernel (new and displaced barcodes)"
                              : "specialised (NVRTC) spec_random_kernel, filter+verify + 16-byte-slot count table (home sector requested a tile ahead), " +
                                    std::to_string(specialised_blocks_per_sm(k)) + " blocks/SM; + random_insert_kernel (new and displaced barcodes)";
     if (!m.params.use_first) ctx.kernel_note += " + random_kernel on the multi-window reads";
@@ -1070,7 +1095,6 @@ int scg_plan_harvest(scg_plan* plan, scg_result** table) {
         if (plan->kind == scg_plan::COMBO) {
             plan->tally.harvest(c, *r);
         } else if (plan->kind == scg_plan::RANDOM) {
-            if (plan->random->wide) throw Error("plans of random barcodes longer than 21 bases cannot be harvested on the device");
             SortedTable sorted;
             plan->table.sorted(c, plan->random->key_len, sorted);
             r->width = plan->random->key_len;
@@ -1099,7 +1123,6 @@ int scg_plan_sorted_table(scg_plan* plan, scg_table** out) {
         if (plan->kind == scg_plan::COMBO) {
             plan->tally.sorted(c, t->table);
         } else if (plan->kind == scg_plan::RANDOM) {
-            if (plan->random->wide) throw Error("random barcodes longer than 21 bases have no sorted device table");
             plan->table.sorted(c, plan->random->key_len, t->table);
         } else {
             throw Error("only combinatorial and random-barcode plans hold a table");
@@ -1122,6 +1145,7 @@ int scg_plan_dense_tally(scg_plan* plan, void** d_matrix, long long* cells) {
 
 long long scg_table_rows(const scg_table* t) { return t ? (long long)t->table.rows : 0; }
 int scg_table_key_len(const scg_table* t) { return t ? t->table.key_len : 0; }
+int scg_table_key_words(const scg_table* t) { return t ? t->table.words() : 0; }
 void* scg_table_keys(const scg_table* t) { return t ? t->table.keys.ptr : nullptr; }
 void* scg_table_counts(const scg_table* t) { return t ? t->table.counts.ptr : nullptr; }
 void scg_table_free(scg_table* t) { delete t; }
@@ -1135,10 +1159,11 @@ int scg_table_from_device(scg_ctx* ctx, const void* d_keys, const void* d_counts
         t->owner = ctx;
         t->table.rows = (size_t)rows;
         t->table.key_len = key_len;
-        t->table.keys.alloc(std::max<size_t>((size_t)rows, 1) * 8, false);
+        const size_t key_bytes = (size_t)rows * 8 * (size_t)t->table.words();
+        t->table.keys.alloc(std::max<size_t>(key_bytes, 8), false);
         t->table.counts.alloc(std::max<size_t>((size_t)rows, 1) * sizeof(uint32_t), false);
         if (rows) {
-            SCG_CUDA_CHECK(cudaMemcpyAsync(t->table.keys.ptr, d_keys, (size_t)rows * 8, cudaMemcpyDeviceToDevice, c.stream));
+            SCG_CUDA_CHECK(cudaMemcpyAsync(t->table.keys.ptr, d_keys, key_bytes, cudaMemcpyDeviceToDevice, c.stream));
             SCG_CUDA_CHECK(cudaMemcpyAsync(t->table.counts.ptr, d_counts, (size_t)rows * sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.stream));
             SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
         }
@@ -1151,6 +1176,10 @@ int scg_table_merge(scg_ctx* ctx, const scg_table* a, const scg_table* b, scg_ta
         Context& c = ctx->impl;
         c.ensure_ready();
         if (!a || !b) throw Error("null table");
+        if (a->table.key_len != b->table.key_len) {
+            throw Error("cannot merge tables of different key lengths (" + std::to_string(a->table.key_len) + " and " +
+                        std::to_string(b->table.key_len) + ")");
+        }
         std::unique_ptr<scg_table> t(new scg_table);
         t->owner = ctx;
         merge_sorted_tables(c, a->table, b->table, t->table);

@@ -503,16 +503,46 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
 // countRandomBarcodes
 // =====================================================================================================================
 #if SPH_KIND == 3
+// barcodes of 22 to 42 bases: 128-bit keys (random_key128) in the wide count table, whose keys and counts are separate arrays
+#define SPH_WIDE (SPH_A_FLEN0 > 21)
+namespace scg {
+namespace sph {
+// bits [START, START + LEN) of a window given as words, LEN <= 64
+template <int START, int LEN, int NW>
+__device__ __forceinline__ unsigned long long window_bits64(const uint32_t (&w)[NW]) {
+    if constexpr (LEN <= 32) {
+        return window_bits<START, LEN>(w);
+    } else {
+        return (unsigned long long)window_bits<START, 32>(w) | ((unsigned long long)window_bits<START + 32, LEN - 32>(w) << 32);
+    }
+}
+} // namespace sph
+} // namespace scg
+
 extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
+#if SPH_WIDE
+    spec_random_kernel(const scg::ReadsDev reads, const scg::CountTable128 table, const uint8_t* __restrict__ odd, long long read_offset,
+#else
     spec_random_kernel(const scg::ReadsDev reads, const scg::CountTable64 table, const uint8_t* __restrict__ odd, long long read_offset,
+#endif
                        scg::OddOutcome* __restrict__ odd_out, unsigned long long* __restrict__ odd_count, int32_t* __restrict__ out_index,
                        const scg::DeferredList def, const scg::SlowList slow, const scg::PartitionedKeys parts) {
     using namespace scg;
     using namespace scg::sph;
     using DA = Dims<TrA>;
     constexpr int KEYLEN = SPH_A_FLEN0;
+#if SPH_WIDE
+    static_assert(KEYLEN <= 42, "barcodes of up to 42 bases fit the 128-bit table");
+    static_assert(!SPH_PARTITIONED, "wide tables are not filled part by part");
+    using KeyT = ulonglong2;
+    using PlaneT = unsigned long long;
+    constexpr unsigned long long KMASK = (1ull << KEYLEN) - 1ull;
+#else
     static_assert(KEYLEN >= 1 && KEYLEN <= 21, "barcodes of up to 21 bases fit the 64-bit table");
+    using KeyT = unsigned long long;
+    using PlaneT = uint32_t;
     constexpr uint32_t KMASK = low_mask(KEYLEN);
+#endif
     constexpr uint32_t BYTES_A = GROUP * DA::TILE_BYTES;
     __shared__ __align__(128) uint32_t stage_a[WARPS][STAGES][GROUP * DA::TILE_WORDS];
     __shared__ __align__(8) unsigned long long bar_all[WARPS][STAGES];
@@ -550,8 +580,9 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
     }
 
     // carried from one tile to the next: the barcode, its home in the count table and what the home's two slots (one
-    // 32-byte sector) held when requested
-    unsigned long long pkey = 0, ppos = 0;
+    // 32-byte sector: two 16-byte slots of a narrow table, two 16-byte keys of a wide one) held when requested
+    KeyT pkey{};
+    unsigned long long ppos = 0;
     uint4 pa = make_uint4(0, 0, 0, 0), pb = make_uint4(0, 0, 0, 0);
     bool pinsert = false;
     const uint32_t region_base = (uint32_t)warp * def.per_warp;
@@ -565,12 +596,13 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
         tiles_here = min(GROUP, ntiles - GROUP * group);
     }
     for (;;) {
-        unsigned long long key = 0;
+        KeyT key{};
         bool insert = false;
         if (have) {
             const uint32_t i = (uint32_t)(group * GROUP + tile_in_group) * TILE + lane;
             const bool inrange = i < n;
-            uint32_t meta = 0, kh = 0, kl = 0, kn = 0;
+            uint32_t meta = 0;
+            PlaneT kh = 0, kl = 0, kn = 0;
             int ncand = 0;
             {
                 Words<TrA::W> R;
@@ -580,9 +612,15 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
                 // the barcode is cut at the FORWARD coordinates on both strands (:106-108; SURVEY 8.1 T9)
                 scan_blocks<TrA, 0>(R, P, inrange, ncand, meta, [&](const uint32_t(&wh)[DA::TW + 1], const uint32_t(&wl)[DA::TW + 1],
                                                                    const uint32_t(&wn)[DA::TW + 1], bool) {
+#if SPH_WIDE
+                    kh = window_bits64<SPH_A_FSTART0, KEYLEN>(wh);
+                    kl = window_bits64<SPH_A_FSTART0, KEYLEN>(wl);
+                    kn = window_bits64<SPH_A_FSTART0, KEYLEN>(wn);
+#else
                     kh = window_bits<SPH_A_FSTART0, KEYLEN>(wh);
                     kl = window_bits<SPH_A_FSTART0, KEYLEN>(wl);
                     kn = window_bits<SPH_A_FSTART0, KEYLEN>(wn);
+#endif
                 });
             }
             if (++tile_in_group == tiles_here) {
@@ -598,7 +636,11 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
             const bool rev = (meta & SM_REV) != 0;
             if (rev) {
                 // reverse complement of the KEYLEN bases; an N stays an N
+#if SPH_WIDE
+                const PlaneT rh = __brevll(kh) >> (64 - KEYLEN), rl = __brevll(kl) >> (64 - KEYLEN), rn = __brevll(kn) >> (64 - KEYLEN);
+#else
                 const uint32_t rh = __brev(kh) >> (32 - KEYLEN), rl = __brev(kl) >> (32 - KEYLEN), rn = __brev(kn) >> (32 - KEYLEN);
+#endif
                 kh = ~rh & KMASK & ~rn;
                 kl = ~rl & KMASK & ~rn;
                 kn = rn;
@@ -614,7 +656,11 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
             }
             slow_append(slow, slowp && inrange, lane, i);
             insert = inrange && counted && !is_odd;
+#if SPH_WIDE
+            key = random_key128(kh, kl, kn);
+#else
             key = random_key64(kh, kl, kn);
+#endif
         }
 
 #if SPH_PARTITIONED
@@ -643,6 +689,26 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
         // sector is counted with one fire-and-forget atomic; one that is not there yet (new, or pushed further along by a
         // collision) goes to the deferred list and the follow-up kernel inserts it -- no compare-and-swap round trip, no
         // probing loop, nothing this warp has to wait for ----
+#if SPH_WIDE
+        {
+            const uint32_t x0 = (uint32_t)pkey.x, x1 = (uint32_t)(pkey.x >> 32), y0 = (uint32_t)pkey.y, y1 = (uint32_t)(pkey.y >> 32);
+            const bool hit_a = pinsert && pa.x == x0 && pa.y == x1 && pa.z == y0 && pa.w == y1;
+            const bool hit_b = pinsert && pb.x == x0 && pb.y == x1 && pb.z == y0 && pb.w == y1;
+            if (hit_a || hit_b) atomicAdd(table.counts + ppos + (hit_a ? 0u : 1u), 1u);
+            const uint32_t entry[4] = { x0, x1, y0, y1 };
+            defer_append<4>(def, region_base, cursor, pinsert && !hit_a && !hit_b, lane, entry);
+        }
+
+        // ---- this tile's barcodes: request their home sectors ----
+        pinsert = insert;
+        pkey = key;
+        if (insert) {
+            ppos = count_home128(table, key);
+            const uint4* __restrict__ home = reinterpret_cast<const uint4*>(table.keys + ppos);
+            pa = __ldcg(home);
+            pb = __ldcg(home + 1);
+        }
+#else
         {
             const unsigned long long ka = (unsigned long long)pa.x | ((unsigned long long)pa.y << 32);
             const unsigned long long kb = (unsigned long long)pb.x | ((unsigned long long)pb.y << 32);
@@ -661,6 +727,7 @@ extern "C" __global__ void __launch_bounds__(128, SPH_MIN_BLOCKS)
             pa = __ldcg(home);
             pb = __ldcg(home + 1);
         }
+#endif
 
         if (!have) break;
 #endif

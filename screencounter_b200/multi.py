@@ -76,8 +76,9 @@ def combine_dense(counts, scalars=(), group=None):
 class _DevView:
     """Zero-copy torch view of device memory this library owns (CUDA array interface)."""
 
-    def __init__(self, ptr, n, typestr):
-        self.__cuda_array_interface__ = {"shape": (int(n),), "typestr": typestr, "data": (int(ptr), False), "version": 2}
+    def __init__(self, ptr, shape, typestr):
+        shape = (int(shape),) if isinstance(shape, (int, np.integer)) else tuple(int(d) for d in shape)
+        self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 2}
 
 
 class DeviceTableOps:
@@ -95,14 +96,16 @@ class DeviceTableOps:
         return h
 
     def views(self, table):
-        """(keys int64, counts int32) torch views of a table's device arrays (keys are below 2^63)."""
+        """(keys int64 of shape (rows, words), counts int32) torch views of a table's device arrays.  A row's words are in
+        the order they sort by (include/scg.h scg_table_keys); every word is below 2^63."""
         import torch
         from ._lib import lib
         n = int(lib().scg_table_rows(table))
+        words = int(lib().scg_table_key_words(table))
         if n == 0:
             dev = torch.device("cuda", torch.cuda.current_device())
-            return torch.empty(0, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.int32, device=dev)
-        keys = torch.as_tensor(_DevView(lib().scg_table_keys(table), n, "<i8"), device="cuda")
+            return torch.empty((0, words), dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.int32, device=dev)
+        keys = torch.as_tensor(_DevView(lib().scg_table_keys(table), (n, words), "<i8"), device="cuda")
         counts = torch.as_tensor(_DevView(lib().scg_table_counts(table), n, "<i4"), device="cuda")
         return keys, counts
 
@@ -116,8 +119,9 @@ class DeviceTableOps:
         from .rcpp import _check
         torch.cuda.current_stream().synchronize()   # the tensors were produced on torch's stream, the copy runs on the library's
         h = C.c_void_p()
+        keys = keys.contiguous()
         _check(self.ctx, lib().scg_table_from_device(self.ctx, C.c_void_p(keys.data_ptr()), C.c_void_p(counts.data_ptr()),
-                                                     C.c_longlong(keys.numel()), int(key_len), C.byref(h)))
+                                                     C.c_longlong(keys.shape[0]), int(key_len), C.byref(h)))
         return h
 
     def merge(self, a, b):
@@ -144,36 +148,55 @@ class DeviceTableOps:
             lib().scg_result_free(h)
 
 
+def _cut(keys, splitters):
+    """Rows of the sorted table `keys` that sort before each splitter row.  Keys of two words per row (random barcodes longer
+    than 21 bases) compare lexicographically: word 0 locates the run of rows that share the splitter's word 0, word 1 the
+    place inside that run."""
+    import torch
+    if keys.dim() == 1:
+        return torch.searchsorted(keys, splitters)
+    w0 = keys[:, 0].contiguous()
+    lo = torch.searchsorted(w0, splitters[:, 0].contiguous())
+    hi = torch.searchsorted(w0, splitters[:, 0].contiguous(), right=True)
+    cuts = [torch.searchsorted(keys[a:b, 1].contiguous(), splitters[j:j + 1, 1].contiguous()) + a
+            for j, (a, b) in enumerate(zip(lo.tolist(), hi.tolist()))]
+    return torch.cat(cuts) if cuts else torch.empty(0, dtype=torch.int64, device=keys.device)
+
+
 def merge_tables_across_ranks(ops, local, group=None, gather_to=0):
     """The sparse exchange described at the top of this file.  `local` is this rank's sorted table (an `ops` handle; it is
-    consumed).  Returns the merged table of ALL ranks on rank `gather_to` (None elsewhere) and a dict of what moved."""
+    consumed).  Returns the merged table of ALL ranks on rank `gather_to` (None elsewhere) and a dict of what moved.
+    `ops.views` gives keys of one int64 per row (a vector, or a (rows, 1) matrix) or of two (a (rows, 2) matrix)."""
     import torch
     dist = _dist()
     world = dist.get_world_size(group)
     rank = dist.get_rank(group)
     keys, counts = ops.views(local)
+    if keys.dim() == 2 and keys.shape[1] == 1:
+        keys = keys.reshape(-1)   # one word per row: the int64 values are the order
+    row = tuple(keys.shape[1:])   # () for one word per row, (2,) for two
     dev = keys.device
     key_len = ops.key_len(local)
     # --- splitters: world - 1 keys at the quantiles of rank 0's table, broadcast ---
-    splitters = torch.zeros(max(world - 1, 1), dtype=torch.int64, device=dev)
-    if rank == 0 and keys.numel() > 0 and world > 1:
-        at = (torch.arange(1, world, device=dev, dtype=torch.int64) * keys.numel()) // world
+    splitters = torch.zeros((max(world - 1, 1),) + row, dtype=torch.int64, device=dev)
+    if rank == 0 and keys.shape[0] > 0 and world > 1:
+        at = (torch.arange(1, world, device=dev, dtype=torch.int64) * keys.shape[0]) // world
         splitters[: world - 1] = keys[at]
-    nrows = torch.tensor([keys.numel()], dtype=torch.int64, device=dev)
+    nrows = torch.tensor([keys.shape[0]], dtype=torch.int64, device=dev)
     dist.broadcast(splitters, src=0, group=group)
     dist.broadcast(nrows, src=0, group=group)
     if int(nrows.item()) == 0:
         splitters.fill_(np.iinfo(np.int64).max)   # rank 0 holds nothing: everything goes to rank 0's range
     # --- cut this rank's table at the splitters (it is sorted: every range is a contiguous slice) ---
-    cuts = torch.searchsorted(keys, splitters[: world - 1]) if world > 1 else torch.empty(0, dtype=torch.int64, device=dev)
+    cuts = _cut(keys, splitters[: world - 1]) if world > 1 else torch.empty(0, dtype=torch.int64, device=dev)
     bounds = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), cuts.to(torch.int64),
-                        torch.tensor([keys.numel()], dtype=torch.int64, device=dev)])
+                        torch.tensor([keys.shape[0]], dtype=torch.int64, device=dev)])
     send_sizes = (bounds[1:] - bounds[:-1]).contiguous()
     recv_sizes = torch.empty_like(send_sizes)
     dist.all_to_all_single(recv_sizes, send_sizes, group=group)
     send_list, recv_list = send_sizes.tolist(), recv_sizes.tolist()
     # --- ONE all-to-all per array: range r of every rank goes to rank r ---
-    rkeys = torch.empty(int(sum(recv_list)), dtype=torch.int64, device=dev)
+    rkeys = torch.empty((int(sum(recv_list)),) + row, dtype=torch.int64, device=dev)
     rcounts = torch.empty(int(sum(recv_list)), dtype=torch.int32, device=dev)
     dist.all_to_all_single(rkeys, keys.contiguous(), output_split_sizes=recv_list, input_split_sizes=send_list, group=group)
     dist.all_to_all_single(rcounts, counts.contiguous(), output_split_sizes=recv_list, input_split_sizes=send_list, group=group)
@@ -195,19 +218,21 @@ def merge_tables_across_ranks(ops, local, group=None, gather_to=0):
     mine = runs[0]
     # --- the ranges, in rank order, are the sorted table of everything: gathered on one rank ---
     mkeys, mcounts = ops.views(mine)
+    mkeys = mkeys.reshape((mkeys.shape[0],) + row)
     sizes = torch.zeros(world, dtype=torch.int64, device=dev)
-    sizes[rank] = mkeys.numel()
+    sizes[rank] = mkeys.shape[0]
     dist.all_reduce(sizes, group=group)
     size_list = sizes.tolist()
-    to_root = [int(mkeys.numel()) if r == gather_to else 0 for r in range(world)]
+    to_root = [int(mkeys.shape[0]) if r == gather_to else 0 for r in range(world)]
     from_all = [int(s) for s in size_list] if rank == gather_to else [0] * world
-    gkeys = torch.empty(int(sum(from_all)), dtype=torch.int64, device=dev)
+    gkeys = torch.empty((int(sum(from_all)),) + row, dtype=torch.int64, device=dev)
     gcounts = torch.empty(int(sum(from_all)), dtype=torch.int32, device=dev)
     dist.all_to_all_single(gkeys, mkeys.contiguous(), output_split_sizes=from_all, input_split_sizes=to_root, group=group)
     dist.all_to_all_single(gcounts, mcounts.contiguous(), output_split_sizes=from_all, input_split_sizes=to_root, group=group)
     ops.free(mine)
+    row_bytes = 8 * (row[0] if row else 1) + 4
     info = {"rows_sent": int(sum(send_list)), "rows_owned_after_merge": int(size_list[rank]), "rows_total": int(sum(size_list)),
-            "bytes_all_to_all": int(sum(send_list)) * 12}
+            "bytes_all_to_all": int(sum(send_list)) * row_bytes}
     if rank != gather_to:
         return None, info
     return ops.from_tensors(gkeys, gcounts, key_len), info
