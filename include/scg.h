@@ -264,8 +264,12 @@ int scg_plan_harvest(scg_plan* plan, scg_result** table);
  *   scg_plan_dense_tally    combinations tallied in a dense n1 x n2 matrix: its device address (else *d_matrix = NULL)
  *   scg_table_key_words     64-bit words per row of the table's keys (1 or 2)
  *   scg_table_from_device   a table from device arrays the caller owns (copied: rows x words keys, rows counts), e.g. rows
- *                           received from another GPU
- *   scg_table_merge         sorted union of two tables, counts of equal keys added; tables of different key_len are refused
+ *                           received from another GPU.  The copy is checked in one device pass and refused (status 1, no
+ *                           table) unless key_len is in 0..42, rows ascend strictly by (word 0, word 1), every 3-bit rank of
+ *                           a barcode is at most 4 with no bits set above the bases a word holds, both halves of a combination
+ *                           are below 2^31, and every count is below 2^31
+ *   scg_table_merge         sorted union of two tables, counts of equal keys added; tables of different key_len are refused.
+ *                           Known limit: a sum is not checked for overflow (the reference's int counters overflow too)
  *   scg_table_render        the table as the file-level calls return it (rows stay on the device until copied) */
 int scg_plan_sorted_table(scg_plan* plan, scg_table** out);
 int scg_plan_dense_tally(scg_plan* plan, void** d_matrix, long long* cells);

@@ -221,6 +221,10 @@ void render_combinations(Context& ctx, const SortedTable& t, DeviceBuffer& keys,
 void device_table_result(Context& ctx, const SortedTable& t, scg_result& out);
 // c = sorted merge of a and b with the counts of equal keys added (a and b sorted ascending, keys unique within each)
 void merge_sorted_tables(Context& ctx, const SortedTable& a, const SortedTable& b, SortedTable& c);
+// throws unless the rows of t (key_len in 0..42) are those of a well-formed SortedTable: strictly ascending, every barcode rank
+// <= 4 and no bits above the bases a word holds, both halves of a combination below 2^31, counts below 2^31 (one device pass;
+// synchronises)
+void validate_sorted_table(Context& ctx, const SortedTable& t);
 
 // column[i] = count of all_keys' row i in t (0 where t lacks the key): one column of a many-files count matrix
 void scatter_table_column(Context& ctx, const SortedTable& all_keys, const SortedTable& t, int32_t* column);

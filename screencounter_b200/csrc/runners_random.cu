@@ -452,6 +452,68 @@ void merge_sorted_tables(Context& ctx, const SortedTable& a, const SortedTable& 
     SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
 }
 
+// What validate_table_kernel found wrong with a table, one bit per kind of fault (messages in validate_sorted_table)
+enum : uint32_t { TABLE_UNSORTED = 1, TABLE_DUPLICATE = 2, TABLE_RANK = 4, TABLE_HIGH_BITS = 8, TABLE_COMBO_INDEX = 16, TABLE_COUNT = 32 };
+
+// faults of one word of a barcode key that holds `groups` (1..21) bases: a 3-bit rank above 4 (the renderer indexes "ACGNT"
+// with it), or bits set above the bases
+__device__ __forceinline__ uint32_t barcode_word_faults(unsigned long long w, int groups) {
+    const unsigned long long used = (1ull << (3 * groups)) - 1;
+    const unsigned long long low = 0x1249249249249249ull & used;   // bit 0 of every group in use
+    uint32_t e = (w & ~used) ? TABLE_HIGH_BITS : 0u;
+    if ((w >> 2) & (w | (w >> 1)) & low) e |= TABLE_RANK;       // bit 2 set and bit 1 or 0 set: 5, 6 or 7
+    return e;
+}
+
+// one row per thread: the row's key and count, and its order against the row before it; faults are or-ed into *err
+__global__ void validate_table_kernel(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ counts, size_t n, int key_len,
+                                      uint32_t* err) {
+    const int words = key_len > 21 ? 2 : 1;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const unsigned long long* row = keys + i * (size_t)words;
+        const unsigned long long k0 = row[0], k1 = words == 2 ? row[1] : 0ull;
+        uint32_t e = 0;
+        if (key_len == 0) {
+            if (k0 & 0x8000000080000000ull) e |= TABLE_COMBO_INDEX;
+        } else {
+            e |= barcode_word_faults(k0, min(key_len, 21));
+            if (words == 2) e |= barcode_word_faults(k1, key_len - 21);
+        }
+        if (counts[i] >> 31) e |= TABLE_COUNT;
+        if (i > 0) {
+            const unsigned long long p0 = row[-words], p1 = words == 2 ? row[-1] : 0ull;
+            if (p0 == k0 && p1 == k1) {
+                e |= TABLE_DUPLICATE;
+            } else if (p0 > k0 || (p0 == k0 && p1 > k1)) {
+                e |= TABLE_UNSORTED;
+            }
+        }
+        if (e) atomicOr(err, e);
+    }
+}
+
+void validate_sorted_table(Context& ctx, const SortedTable& t) {
+    if (t.rows == 0) return;
+    DeviceBuffer d_err;
+    d_err.alloc(sizeof(uint32_t), true);
+    validate_table_kernel<<<fill_grid(ctx, t.rows), 256, 0, ctx.stream>>>(t.keys.as<unsigned long long>(), t.counts.as<uint32_t>(), t.rows, t.key_len,
+                                                                         d_err.as<uint32_t>());
+    SCG_CUDA_CHECK(cudaGetLastError());
+    ++ctx.launches;
+    uint32_t err = 0;
+    SCG_CUDA_CHECK(cudaMemcpyAsync(&err, d_err.ptr, sizeof err, cudaMemcpyDeviceToHost, ctx.stream));
+    SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    if (!err) return;
+    static const char* const what[] = { "rows are not in ascending key order", "a key appears in two rows",
+                                        "a key holds a base rank above 4", "a key has bits set beyond its key length",
+                                        "a combination index is 2^31 or more", "a count is 2^31 or more" };
+    std::string msg = "malformed sorted table:";
+    for (int b = 0; b < 6; ++b) {
+        if (err & (1u << b)) msg += std::string(msg.back() == ':' ? " " : "; ") + what[b];
+    }
+    throw Error(msg);
+}
+
 // column[i] = count of all_keys[i] in table t, 0 where t does not hold the key (every key of t is in all_keys)
 template <class K>
 __global__ void scatter_column_kernel(const K* __restrict__ uk, size_t nu, const K* __restrict__ tk, const uint32_t* __restrict__ tc, size_t nt,

@@ -1155,6 +1155,7 @@ int scg_table_from_device(scg_ctx* ctx, const void* d_keys, const void* d_counts
         Context& c = ctx->impl;
         c.ensure_ready();
         if (rows < 0) throw Error("negative number of rows");
+        if (key_len < 0 || key_len > 42) throw Error("key length " + std::to_string(key_len) + " is outside 0..42");
         std::unique_ptr<scg_table> t(new scg_table);
         t->owner = ctx;
         t->table.rows = (size_t)rows;
@@ -1165,8 +1166,10 @@ int scg_table_from_device(scg_ctx* ctx, const void* d_keys, const void* d_counts
         if (rows) {
             SCG_CUDA_CHECK(cudaMemcpyAsync(t->table.keys.ptr, d_keys, key_bytes, cudaMemcpyDeviceToDevice, c.stream));
             SCG_CUDA_CHECK(cudaMemcpyAsync(t->table.counts.ptr, d_counts, (size_t)rows * sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.stream));
-            SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
         }
+        // foreign rows: the merge's binary searches and the renderer rely on what a table promises (include/scg.h);
+        // synchronises the copies; a refused table is freed with t
+        validate_sorted_table(c, t->table);
         *out = t.release();
     });
 }

@@ -85,8 +85,12 @@ class DeviceTableOps:
     """The table operations of the sparse exchange, on the device through the C ABI (include/scg.h scg_table_*)."""
 
     def __init__(self, device=None):
-        from .rcpp import context
+        from .rcpp import context, default_device
         self.ctx = context(device)
+        if device is None:
+            device = default_device()
+        # the device the context's tables live on: the first of a multi-device context
+        self.device = int(device[0] if isinstance(device, (list, tuple)) else device)
 
     def from_plan(self, plan):
         from ._lib import lib
@@ -103,7 +107,7 @@ class DeviceTableOps:
         n = int(lib().scg_table_rows(table))
         words = int(lib().scg_table_key_words(table))
         if n == 0:
-            dev = torch.device("cuda", torch.cuda.current_device())
+            dev = torch.device("cuda", self.device)
             return torch.empty((0, words), dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.int32, device=dev)
         keys = torch.as_tensor(_DevView(lib().scg_table_keys(table), (n, words), "<i8"), device="cuda")
         counts = torch.as_tensor(_DevView(lib().scg_table_counts(table), n, "<i4"), device="cuda")
@@ -114,12 +118,26 @@ class DeviceTableOps:
         return int(lib().scg_table_key_len(table))
 
     def from_tensors(self, keys, counts, key_len):
+        """A table copied from `keys` (int64, (rows, words), or (rows,) when a row has one word) and `counts` (int32, (rows,)),
+        both on this context's device.  The library refuses rows that are not a sorted table (include/scg.h)."""
         import torch
         from ._lib import lib
         from .rcpp import _check
-        torch.cuda.current_stream().synchronize()   # the tensors were produced on torch's stream, the copy runs on the library's
+        dev = torch.device("cuda", self.device)
+        words = 2 if int(key_len) > 21 else 1
+        if not isinstance(keys, torch.Tensor) or keys.dtype != torch.int64 or keys.device != dev:
+            raise ValueError("table keys must be an int64 tensor on %s" % dev)
+        if not isinstance(counts, torch.Tensor) or counts.dtype != torch.int32 or counts.device != dev:
+            raise ValueError("table counts must be an int32 tensor on %s" % dev)
+        if not (keys.dim() == 2 and keys.shape[1] == words or keys.dim() == 1 and words == 1):
+            raise ValueError("table keys of key length %d must have shape (rows, %d)%s, not %s"
+                             % (key_len, words, " or (rows,)" if words == 1 else "", tuple(keys.shape)))
+        rows = keys.shape[0]
+        if counts.dim() != 1 or counts.shape[0] != rows:
+            raise ValueError("table counts must have shape (%d,), not %s" % (rows, tuple(counts.shape)))
+        keys, counts = keys.contiguous(), counts.contiguous()
+        torch.cuda.current_stream(dev).synchronize()   # the tensors were produced on torch's stream, the copy runs on the library's
         h = C.c_void_p()
-        keys = keys.contiguous()
         _check(self.ctx, lib().scg_table_from_device(self.ctx, C.c_void_p(keys.data_ptr()), C.c_void_p(counts.data_ptr()),
                                                      C.c_longlong(keys.shape[0]), int(key_len), C.byref(h)))
         return h

@@ -22,10 +22,15 @@ class ScreenCounterError(RuntimeError):
 _local = threading.local()
 
 
+def default_device():
+    """The device of a context asked for without one: SCG_DEVICE, else LOCAL_RANK, else 0."""
+    return int(os.environ.get("SCG_DEVICE", os.environ.get("LOCAL_RANK", "0")))
+
+
 def context(device=None):
     """Per-thread, per-device context (CUDA is initialised lazily by the first counting call)."""
     if device is None:
-        device = int(os.environ.get("SCG_DEVICE", os.environ.get("LOCAL_RANK", "0")))
+        device = default_device()
     cache = getattr(_local, "ctx", None)
     if cache is None:
         cache = _local.ctx = {}
