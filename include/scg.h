@@ -94,7 +94,7 @@ int scg_count_single(scg_ctx* ctx, const scg_source* src, const char* constant, 
                      int32_t* counts, int32_t* total, scg_result** trace);
 
 /* replaces count_random_barcodes, src/count_random_barcodes.cpp:41-60.
- * table: distinct barcodes (strings) + frequencies. */
+ * table: distinct barcodes (strings) + frequencies.  Barcodes of any length a template holds are counted on the device. */
 int scg_count_random(scg_ctx* ctx, const scg_source* src, const char* constant, int strand,
                      int mismatches, int use_first, int nthreads,
                      scg_result** table, int32_t* total);
@@ -260,6 +260,11 @@ int scg_plan_harvest(scg_plan* plan, scg_result** table);
  *                              bases 21..key_len-1 in the same convention.
  * Every word is below 2^63, so signed 64-bit views keep the order.  counts: unsigned 32-bit, one per row.  key_len > 0 marks
  * random barcodes of that length; the number of words follows from it (two when key_len > 21).
+ * These tables hold random barcodes of at most 42 bases.  Longer barcodes (43 bases up to what a 256-character template
+ * holds) are counted by scg_count_random, scg_count_random_many and the random plans (scg_plan_harvest) like any others, in a
+ * device table of ceil(key_len / 21) words per row in the same convention, but that table is not handed out here:
+ * scg_plan_sorted_table refuses a plan of longer barcodes ("sorted tables hold random barcodes of at most 42 bases"), so no
+ * table leaves that scg_table_from_device could not take back.
  *   scg_plan_sorted_table   the plan's tally, sorted (synchronises the device)
  *   scg_plan_dense_tally    combinations tallied in a dense n1 x n2 matrix: its device address (else *d_matrix = NULL)
  *   scg_table_key_words     64-bit words per row of the table's keys (1 or 2)

@@ -13,8 +13,8 @@
 
 namespace scg {
 
-// 64-bit words per row of a sorted table's keys (SortedTable): two for random barcodes longer than 21 bases, one otherwise
-inline int table_key_words(int key_len) { return key_len > 21 ? 2 : 1; }
+// 64-bit words per row of a sorted table's keys (SortedTable): one per 21 bases of a random barcode, one for combinations
+inline int table_key_words(int key_len) { return key_len > 0 ? (key_len + 20) / 21 : 1; }
 
 std::string& creation_error();   // message of a failed scg_ctx_create
 
@@ -176,13 +176,11 @@ void launch_single(Context& ctx, const ReadsDev& reads, const SingleMatcher& m, 
                    uint32_t* d_info, cudaStream_t stream);
 
 // A sparse result resident on the device, sorted: what scg_result hands out on demand (scg_result_copy_table) and what the
-// multi-GPU merge exchanges.  keys: table_key_words(key_len) 64-bit words per row, row-major, rows ascending by (word 0,
-// word 1):
+// multi-GPU merge exchanges.  keys: table_key_words(key_len) 64-bit words per row, row-major, rows ascending by word 0, 1, ...:
 //   combinations            one word, first << 32 | second;
-//   random barcodes <= 21   one word, three bits per base in text order (A=0 < C=1 < G=2 < N=3 < T=4), first base most
-//                           significant;
-//   random barcodes 22..42  two words: word 0 = the ranks of bases 0..20 (the one-word key of the first 21 bases), word 1 =
-//                           the ranks of bases 21..key_len-1 in the same convention.
+//   random barcodes         ceil(key_len / 21) words: word w = the ranks of bases [21w, min(21w + 21, key_len)), three bits per
+//                           base in text order (A=0 < C=1 < G=2 < N=3 < T=4), first base most significant, right-aligned (so
+//                           one word up to 21 bases, two up to 42, the layout of include/scg.h).
 // Every word is below 2^63, so int64 views keep the order.
 struct SortedTable {
     DeviceBuffer keys, counts;   // unsigned long long[rows * words()], uint32_t[rows]
@@ -191,26 +189,34 @@ struct SortedTable {
     int words() const { return table_key_words(key_len); }
 };
 
-// Device count table (libdev.hpp: 16-byte slots for 64-bit keys, separate arrays for 128-bit keys).  Sized for a load
-// factor of at most 1/2 of the keys it may hold; how many distinct keys it holds is tracked ON THE DEVICE (a counter bumped
-// by every first insert), so the table follows the number of distinct keys, not the number of reads.
+// Device count table (libdev.hpp: 16-byte slots for 64-bit keys, separate arrays for 128-bit keys, tags + counts + a key
+// store for keys of three words or more).  Sized for a load factor of at most 1/2 of the keys it may hold; how many distinct
+// keys it holds is tracked ON THE DEVICE (a counter bumped by every first insert), so the table follows the number of
+// distinct keys, not the number of reads.
 struct CountTable {
     bool wide = false;
-    DeviceBuffer slots;    // narrow: CountSlot[capacity]; wide: ulonglong2[capacity]
-    DeviceBuffer counts;   // wide only: uint32_t[capacity]
+    int long_words = 0;    // > 0: a long-key table (CountTableLong) of this many text-order words per key
+    DeviceBuffer slots;    // narrow: CountSlot[capacity]; wide: ulonglong2[capacity]; long: tags[capacity]
+    DeviceBuffer counts;   // wide and long: uint32_t[capacity]
+    DeviceBuffer keys;     // long only: key store, long_words words per slot
+    DeviceBuffer staging, fresh, fresh_count;   // long only: per launch (CountTableLong), sized by view_long()
+    size_t staging_rows = 0;
     DeviceBuffer live;     // device: [0] distinct keys inserted, [1] overflow flag
     size_t capacity = 0;
     long long live_known = 0;   // distinct keys at the last read-back
     long long pending = 0;      // inserts launched since (each may be a new key)
     bool fixed = false;         // sized by the caller (resident plans): ensure() never grows it
-    void init(Context& ctx, bool wide128, size_t initial);
+    void init(Context& ctx, bool wide128, size_t initial, int long_words = 0);
     void reset(Context& ctx, cudaStream_t stream);            // empties the table, asynchronously
     void ensure(Context& ctx, long long upcoming_inserts);    // keeps (distinct keys + upcoming) <= capacity / 2; may synchronise
     void check_overflow(Context& ctx);                        // throws when inserts were dropped (synchronises)
     CountTable64 view64() const;
     CountTable128 view128() const;
+    CountTableLong view_long(size_t rows);                   // with staging room for a launch over `rows` reads
+    void promote_fresh(Context& ctx, cudaStream_t stream);  // a launch's fresh keys into the key store, its fresh list emptied
     // live entries sorted on the device (SortedTable).  key_len > 0: keys are random barcodes (random_key64, or random_key128
-    // in a wide table), re-coded to text order before the sort; key_len == 0: sorted as they are (combinations).
+    // in a wide table), re-coded to text order before the sort, or the text-order words of a long table; key_len == 0: sorted
+    // as they are (combinations).
     void sorted(Context& ctx, int key_len, SortedTable& out);
 };
 

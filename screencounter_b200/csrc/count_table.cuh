@@ -101,6 +101,100 @@ __device__ __forceinline__ void count_insert128(const CountTable128& t, ulonglon
     if (count_add128(t, key, add)) atomicAdd(t.live, 1ull);
 }
 
+// ---- keys of three words or more (CountTableLong) ----
+// tag: bits 34..63 the key's fingerprint (the top bits of its hash), bit 33 set in every occupied slot, bit 32 while the key
+// is FRESH (its words are still in the staging row of bits 0..31)
+constexpr unsigned long long LONG_PRINT = ~((1ull << 34) - 1);
+constexpr unsigned long long LONG_OCCUPIED = 1ull << 33;
+constexpr unsigned long long LONG_FRESH = 1ull << 32;
+constexpr unsigned long long LONG_ROW = 0xFFFFFFFFull;
+
+// hash of a key word by word (long_hash_step over the words from a seed of 0, then long_hash_final)
+__device__ __forceinline__ unsigned long long long_hash_step(unsigned long long h, unsigned long long word) {
+    h = (h ^ word) * 0x9E3779B97F4A7C15ull;
+    return h ^ (h >> 29);
+}
+__device__ __forceinline__ unsigned long long long_hash_final(unsigned long long h) {
+    h = (h ^ (h >> 32)) * 0xD6E8FEB86659FD93ull;
+    return h ^ (h >> 32);
+}
+__device__ __forceinline__ unsigned long long long_key_hash(const unsigned long long* key, int words) {
+    unsigned long long h = 0;
+    for (int w = 0; w < words; ++w) h = long_hash_step(h, key[w]);
+    return long_hash_final(h);
+}
+
+// a tag as every thread of the grid sees it (no stale copy in L1)
+__device__ __forceinline__ unsigned long long load_tag(const unsigned long long* p) {
+    unsigned long long v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+__device__ __forceinline__ bool long_rows_equal(const unsigned long long* a, const unsigned long long* b, int words) {
+    for (int w = 0; w < words; ++w) {
+        if (__ldcg(a + w) != __ldcg(b + w)) return false;
+    }
+    return true;
+}
+
+// Adds `add` to the count of the key in staging row `row` (hash h), claiming a slot when the key is new (*fresh).  Returns the
+// slot, or ~0 when the probe limit was reached (the overflow flag is raised and nothing is counted).  The row must have been
+// written and fenced (__threadfence) before the call: a claim publishes it to every other thread.
+__device__ __forceinline__ unsigned long long count_add_long(const CountTableLong& t, unsigned long long h, unsigned long long row, uint32_t add,
+                                                             bool& fresh) {
+    const unsigned long long words = (unsigned long long)t.words;
+    const unsigned long long* own = t.staging + row * words;
+    const unsigned long long print = h & LONG_PRINT;
+    unsigned long long pos = h & t.mask & ~1ull;
+    fresh = false;
+    for (unsigned long long probes = 0;; ++probes) {
+        unsigned long long tag = load_tag(t.tags + pos);
+        if (tag == 0) {
+            tag = atomicCAS(t.tags + pos, 0ull, print | LONG_OCCUPIED | LONG_FRESH | row);
+            if (tag == 0) {
+                fresh = true;
+                break;
+            }
+        }
+        if ((tag & LONG_PRINT) == print) {
+            const unsigned long long* other;
+            if (tag & LONG_FRESH) {
+                __threadfence();   // pairs with the claimer's fence between writing its row and publishing the tag
+                other = t.staging + (tag & LONG_ROW) * words;
+            } else {
+                other = t.keys + pos * words;
+            }
+            if (long_rows_equal(own, other, t.words)) break;
+        }
+        if (probes >= COUNT_MAX_PROBES || probes > t.mask) {
+            atomicExch(t.live + 1, 1ull);
+            return ~0ull;
+        }
+        pos = (pos + 1) & t.mask;
+    }
+    atomicAdd(t.counts + pos, add);
+    return pos;
+}
+
+// count_add_long of one read's key, the slots claimed by the warp listed in t.fresh and counted in t.live[0] with one atomic
+// each per warp
+__device__ __forceinline__ void count_insert_long(const CountTableLong& t, unsigned long long h, unsigned long long row) {
+    bool fresh;
+    const unsigned long long pos = count_add_long(t, h, row, 1u, fresh);
+    const uint32_t active = __activemask();
+    const uint32_t m = __ballot_sync(active, fresh);
+    if (!m) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) {
+        base = atomicAdd(t.fresh_count, (unsigned long long)__popc(m));
+        atomicAdd(t.live, (unsigned long long)__popc(m));
+    }
+    base = __shfl_sync(active, base, leader);
+    if (fresh) t.fresh[base + __popc(m & ((1u << lane) - 1u))] = pos;
+}
+
 __device__ __forceinline__ void combo_count(const ComboSink& k, int id0, int id1) {
     if (k.dense) {
         atomicAdd(k.dense + (size_t)id0 * k.n2 + id1, 1);

@@ -131,8 +131,37 @@ __global__ void __launch_bounds__(128) single_kernel(ReadsDev reads, SingleParam
 // -------------------------------------------------------------------------------------------
 
 
+// A key of more than 42 bases as the text-order words of SortedTable (three bits a base, 21 bases a word, the first base most
+// significant) into its staging row; returns the key's hash (long_key_hash of those words).
+template <int KW>
+__device__ __forceinline__ unsigned long long store_long_key(const Key<KW>& key, int len, unsigned long long* row) {
+    unsigned long long h = 0, s = 0;
+    int in_word = 0, w = 0;
+#pragma unroll
+    for (int pw = 0; pw < KW; ++pw) {
+        const uint32_t H = key.h[pw], L = key.l[pw], N = key.n[pw];
+        const int end = min(32, len - 32 * pw);
+        for (int j = 0; j < end; ++j) {
+            const uint32_t code = (((H >> j) & 1u) << 1) | ((L >> j) & 1u);
+            const uint32_t rank = ((N >> j) & 1u) ? 3u : (code == 3u ? 4u : code);
+            s = (s << 3) | rank;
+            if (++in_word == 21) {
+                row[w++] = s;
+                h = long_hash_step(h, s);
+                s = 0;
+                in_word = 0;
+            }
+        }
+    }
+    if (in_word) {
+        row[w] = s;
+        h = long_hash_step(h, s);
+    }
+    return long_hash_final(h);
+}
+
 template <int CB, int KW>
-__global__ void __launch_bounds__(128) random_kernel(ReadsDev reads, RandomParams P, CountTable64 t64, CountTable128 t128,
+__global__ void __launch_bounds__(128) random_kernel(ReadsDev reads, RandomParams P, CountTable64 t64, CountTable128 t128, CountTableLong tl,
                                                      const uint8_t* __restrict__ odd, long long read_offset,
                                                      OddOutcome* __restrict__ odd_out, unsigned long long* __restrict__ odd_count,
                                                      int32_t* __restrict__ out_index, ReadList visit) {
@@ -194,6 +223,11 @@ __global__ void __launch_bounds__(128) random_kernel(ReadsDev reads, RandomParam
                     if (best_rev) key_revcomp<KW>(key, P.key_len);
                     if (KW == 1 && P.key_len <= 21) {
                         count_insert64(t64, random_key64(key.h[0], key.l[0], key.n[0]), 1u);
+                    } else if (KW > 1 && P.key_len > 42) {
+                        // the key's row of the staging buffer is read i of this launch; written before the probe (CountTableLong)
+                        const unsigned long long h = store_long_key<KW>(key, P.key_len, tl.staging + (unsigned long long)i * (unsigned)tl.words);
+                        __threadfence();
+                        count_insert_long(tl, h, (unsigned long long)i);
                     } else {
                         // up to 42 bases: H, L, N in 42-bit fields of a 128-bit word
                         unsigned long long H = key.h[0], L = key.l[0], N = key.n[0];

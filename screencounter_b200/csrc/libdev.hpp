@@ -86,6 +86,23 @@ struct CountTable128 {
     unsigned long long mask;
     unsigned long long* live;
 };
+// Keys of more than two words (random barcodes of 43 bases or more, `words` text-order words: SortedTable's layout): a tag
+// word per slot (0 = empty; else fingerprint | LONG_OCCUPIED, and while the key is FRESH also LONG_FRESH | its staging row),
+// a count per slot and a key store of `words` words per slot.  A counting kernel writes every key to its own staging row
+// before it probes, so a slot is claimed with ONE compare-and-swap of its tag and nobody ever waits for another thread's key
+// to appear: a FRESH slot is compared against the staging row its tag names, a RESIDENT one against the key store.  A
+// follow-up kernel moves the fresh rows (their slots listed in `fresh`) to the key store before the staging rows are reused.
+struct CountTableLong {
+    unsigned long long* tags;
+    uint32_t* counts;
+    unsigned long long* keys;          // words per slot
+    unsigned long long* staging;       // words per read of the launch, indexed by read
+    unsigned long long* fresh;         // slots claimed by the launch
+    unsigned long long* fresh_count;
+    unsigned long long mask;
+    unsigned long long* live;
+    int words;
+};
 // slot of a key: one 64-bit multiply, the halves folded (the low half alone only mixes upwards)
 SCG_HD unsigned long long count_hash(unsigned long long key) {
     const unsigned long long x = key * 0x9E3779B97F4A7C15ull;

@@ -349,19 +349,20 @@ struct RandomMatcher {
     RandomParams params;
     int key_len = 0;
     bool wide = false;   // barcodes of 22 to 42 bases: 128-bit table keys
+    int long_words = 0;  // barcodes of 43 bases or more: a long-key table of this many words per key (CountTableLong)
 
     void prepare(const std::string& constant, int strand, int mismatches, bool use_first) {
         tmpl = TemplateSpec(constant, strand);
         // the reference dereferences variable_regions()[0] unconditionally (handlers/RandomBarcodeSingleEnd.hpp:93-96, :212-214)
         if (tmpl.fwd_regions.empty()) throw Error("expected at least one variable region in the constant template");
         key_len = tmpl.fwd_regions[0].end - tmpl.fwd_regions[0].start;
-        if (key_len > 42) throw Error("random barcode regions longer than 42 bp are not supported by this engine");
         std::memset(&params, 0, sizeof params);
         params.spec = tmpl.scan_spec(mismatches);
         params.max_mm = mismatches;
         params.use_first = use_first ? 1 : 0;
         params.key_len = key_len;
-        wide = key_len > 21;
+        wide = key_len > 21 && key_len <= 42;
+        long_words = key_len > 42 ? table_key_words(key_len) : 0;
     }
 };
 

@@ -47,6 +47,42 @@ __global__ void rehash128_kernel(const ulonglong2* keys, const uint32_t* counts,
     }
 }
 
+// re-insert the entries of an old long-key table (every one RESIDENT: keys distinct, so only empty slots are claimed)
+__global__ void rehash_long_kernel(const unsigned long long* tags, const uint32_t* counts, const unsigned long long* keys, size_t n,
+                                   CountTableLong dst) {
+    const size_t words = (size_t)dst.words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        if (!tags[i]) continue;
+        const unsigned long long* key = keys + i * words;
+        const unsigned long long h = long_key_hash(key, dst.words);
+        unsigned long long pos = h & dst.mask & ~1ull;
+        for (unsigned long long probes = 0;; ++probes) {
+            if (atomicCAS(dst.tags + pos, 0ull, (h & LONG_PRINT) | LONG_OCCUPIED) == 0) break;
+            if (probes > dst.mask) {
+                atomicExch(dst.live + 1, 1ull);
+                return;
+            }
+            pos = (pos + 1) & dst.mask;
+        }
+        for (size_t w = 0; w < words; ++w) dst.keys[pos * words + w] = key[w];
+        dst.counts[pos] = counts[i];
+        atomicAdd(dst.live, 1ull);
+    }
+}
+
+// the slots a counting launch claimed: their keys from the staging rows into the key store, their tags RESIDENT
+__global__ void promote_fresh_kernel(CountTableLong t) {
+    const unsigned long long n = *t.fresh_count;
+    const size_t words = (size_t)t.words;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned long long pos = t.fresh[i];
+        const unsigned long long tag = t.tags[pos];
+        const unsigned long long* row = t.staging + (tag & LONG_ROW) * words;
+        for (size_t w = 0; w < words; ++w) t.keys[pos * words + w] = row[w];
+        t.tags[pos] = tag & (LONG_PRINT | LONG_OCCUPIED);
+    }
+}
+
 // Rank of every base in the byte order of its letter (A < C < G < N < T, what R's order() sees,
 // R/countRandomBarcodes.R:73), three bits per base, first base most significant: sorting these integers sorts the
 // barcodes as text.  Bases [from, to) of the planes H, L, N (bit b = base b).
@@ -133,21 +169,76 @@ __global__ void unshift_word1_kernel(WideKey* keys, size_t n, int shift1) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) keys[i].w1 >>= shift1;
 }
 
+// compact the live entries of a long-key table (keys already in text order), one atomic per warp
+__global__ void compact_long_kernel(const unsigned long long* tags, const uint32_t* counts, const unsigned long long* keys, size_t n, int words,
+                                    unsigned long long* out_keys, uint32_t* out_counts, unsigned long long* cursor) {
+    const int lane = threadIdx.x & 31;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    const size_t rounds = (n + stride - 1) / stride;
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    for (size_t r = 0; r < rounds; ++r, i += stride) {
+        const bool livep = i < n && tags[i] != 0;
+        const uint32_t m = __ballot_sync(0xFFFFFFFFu, livep);
+        if (!m) continue;
+        unsigned long long base = 0;
+        const int leader = __ffs(m) - 1;
+        if (lane == leader) base = atomicAdd(cursor, (unsigned long long)__popc(m));
+        base = __shfl_sync(0xFFFFFFFFu, base, leader);
+        if (livep) {
+            const unsigned long long at = base + __popc(m & ((1u << lane) - 1u));
+            for (int w = 0; w < words; ++w) out_keys[at * words + w] = keys[i * words + w];
+            out_counts[at] = counts[i];
+        }
+    }
+}
+
+// LSD sort of a long-key table: word w of every row, in the order of the permutation so far
+__global__ void gather_word_kernel(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ perm, size_t n, int words, int w,
+                                   unsigned long long* __restrict__ out) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        out[i] = keys[(size_t)perm[i] * words + w];
+    }
+}
+
+__global__ void iota_kernel(uint32_t* p, size_t n) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = (uint32_t)i;
+}
+
+// rows and counts in the order of the finished permutation
+__global__ void gather_rows_kernel(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ counts, const uint32_t* __restrict__ perm,
+                                   size_t n, int words, unsigned long long* __restrict__ out_keys, uint32_t* __restrict__ out_counts) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t from = perm[i];
+        for (int w = 0; w < words; ++w) out_keys[i * words + w] = keys[from * words + w];
+        out_counts[i] = counts[from];
+    }
+}
+
 static int fill_grid(Context& ctx, size_t n) { return (int)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)ctx.sm_count * 32)); }
 
-void CountTable::init(Context& ctx, bool wide128, size_t initial) {
+void CountTable::init(Context& ctx, bool wide128, size_t initial, int nwords) {
     wide = wide128;
+    long_words = nwords;
     size_t cap = 1024;
     while (cap < initial && cap < (1ull << 33)) cap <<= 1;
     capacity = cap;
-    slots.alloc(capacity * 16, false);
-    if (wide) counts.alloc(capacity * sizeof(uint32_t), false);
+    if (long_words) {
+        slots.alloc(capacity * sizeof(unsigned long long), false);
+        keys.alloc(capacity * (size_t)long_words * sizeof(unsigned long long), false);
+        fresh_count.alloc(sizeof(unsigned long long), true);
+    } else {
+        slots.alloc(capacity * 16, false);
+    }
+    if (wide || long_words) counts.alloc(capacity * sizeof(uint32_t), false);
     live.alloc(2 * sizeof(unsigned long long), false);
     reset(ctx, ctx.stream);
 }
 
 void CountTable::reset(Context& ctx, cudaStream_t stream) {
-    if (wide) {
+    if (long_words) {
+        SCG_CUDA_CHECK(cudaMemsetAsync(slots.ptr, 0, capacity * sizeof(unsigned long long), stream));
+        SCG_CUDA_CHECK(cudaMemsetAsync(counts.ptr, 0, capacity * sizeof(uint32_t), stream));
+    } else if (wide) {
         fill_u64_kernel<<<fill_grid(ctx, capacity * 2), 256, 0, stream>>>(slots.as<unsigned long long>(), ~0ull, capacity * 2);
         SCG_CUDA_CHECK(cudaMemsetAsync(counts.ptr, 0, capacity * sizeof(uint32_t), stream));
     } else {
@@ -177,6 +268,33 @@ CountTable128 CountTable::view128() const {
     return v;
 }
 
+CountTableLong CountTable::view_long(size_t rows) {
+    if (rows > staging_rows) {
+        staging.alloc(rows * (size_t)long_words * sizeof(unsigned long long), false);
+        fresh.alloc(rows * sizeof(unsigned long long), false);
+        staging_rows = rows;
+    }
+    CountTableLong v;
+    v.tags = slots.as<unsigned long long>();
+    v.counts = counts.as<uint32_t>();
+    v.keys = keys.as<unsigned long long>();
+    v.staging = staging.as<unsigned long long>();
+    v.fresh = fresh.as<unsigned long long>();
+    v.fresh_count = fresh_count.as<unsigned long long>();
+    v.mask = capacity - 1;
+    v.live = live.as<unsigned long long>();
+    v.words = long_words;
+    return v;
+}
+
+void CountTable::promote_fresh(Context& ctx, cudaStream_t stream) {
+    promote_fresh_kernel<<<ctx.sm_count * 4, 256, 0, stream>>>(view_long(0));
+    SCG_CUDA_CHECK(cudaGetLastError());
+    SCG_CUDA_CHECK(cudaMemsetAsync(fresh_count.ptr, 0, sizeof(unsigned long long), stream));
+    ++ctx.launches;
+    ++ctx.timing.launches;
+}
+
 void CountTable::check_overflow(Context& ctx) {
     unsigned long long state[2] = { 0, 0 };
     SCG_CUDA_CHECK(cudaMemcpyAsync(state, live.ptr, sizeof state, cudaMemcpyDeviceToHost, ctx.stream));
@@ -201,10 +319,19 @@ void CountTable::ensure(Context& ctx, long long upcoming) {
             size_t ncap = capacity * 2;
             while (ncap < need) ncap *= 2;
             if (ncap > (1ull << 34)) throw Error("the device count table would exceed 2^34 slots");
-            DeviceBuffer nslots, ncounts, nlive;
-            nslots.alloc(ncap * 16, false);
+            DeviceBuffer nslots, ncounts, nkeys, nlive;
+            nslots.alloc(ncap * (long_words ? sizeof(unsigned long long) : 16), false);
             nlive.alloc(2 * sizeof(unsigned long long), true);
-            if (wide) {
+            if (long_words) {
+                const size_t words = (size_t)long_words;
+                nkeys.alloc(ncap * words * sizeof(unsigned long long), false);
+                ncounts.alloc(ncap * sizeof(uint32_t), true);
+                SCG_CUDA_CHECK(cudaMemsetAsync(nslots.ptr, 0, ncap * sizeof(unsigned long long), ctx.stream));
+                CountTableLong dst{ nslots.as<unsigned long long>(), ncounts.as<uint32_t>(), nkeys.as<unsigned long long>(), nullptr, nullptr, nullptr,
+                                    ncap - 1, nlive.as<unsigned long long>(), long_words };
+                rehash_long_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<unsigned long long>(), counts.as<uint32_t>(),
+                                                                                   keys.as<unsigned long long>(), capacity, dst);
+            } else if (wide) {
                 ncounts.alloc(ncap * sizeof(uint32_t), true);
                 fill_u64_kernel<<<fill_grid(ctx, ncap * 2), 256, 0, ctx.stream>>>(nslots.as<unsigned long long>(), ~0ull, ncap * 2);
                 CountTable128 dst{ nslots.as<ulonglong2>(), ncounts.as<uint32_t>(), ncap - 1, nlive.as<unsigned long long>() };
@@ -219,6 +346,7 @@ void CountTable::ensure(Context& ctx, long long upcoming) {
             SCG_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
             slots = std::move(nslots);
             counts = std::move(ncounts);
+            if (long_words) keys = std::move(nkeys);
             live = std::move(nlive);
             capacity = ncap;
         }
@@ -228,7 +356,10 @@ void CountTable::ensure(Context& ctx, long long upcoming) {
 
 // Live entries as (key, count) sorted by key ON THE DEVICE (radix sort), left there in the layout of SortedTable.
 void CountTable::sorted(Context& ctx, int key_len, SortedTable& out) {
-    if (wide != (table_key_words(key_len) == 2)) throw Error("internal error: count table and key length disagree on the key width");
+    const int words = table_key_words(key_len);
+    if (wide != (words == 2) || (long_words != 0) != (words > 2) || (long_words && long_words != words)) {
+        throw Error("internal error: count table and key length disagree on the key width");
+    }
     check_overflow(ctx);
     const size_t nlive = (size_t)live_known;
     out.rows = nlive;
@@ -242,7 +373,36 @@ void CountTable::sorted(Context& ctx, int key_len, SortedTable& out) {
     d_counts.alloc(nlive * sizeof(uint32_t), false);
     d_cursor.alloc(sizeof(unsigned long long), true);
     size_t temp_bytes = 0;
-    if (wide) {
+    if (long_words) {
+        // LSD over the words, last word first: a stable radix sort of each word's 3 * (bases in it) bits carries the permutation
+        if (nlive >= (1ull << 32)) throw Error("long-key tables of 2^32 rows or more cannot be sorted");
+        compact_long_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<unsigned long long>(), counts.as<uint32_t>(),
+                                                                             keys.as<unsigned long long>(), capacity, words, d_keys.as<unsigned long long>(),
+                                                                             d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
+        SCG_CUDA_CHECK(cudaGetLastError());
+        DeviceBuffer word_in, word_out, perm_in, perm_out;
+        word_in.alloc(nlive * sizeof(unsigned long long), false);
+        word_out.alloc(nlive * sizeof(unsigned long long), false);
+        perm_in.alloc(nlive * sizeof(uint32_t), false);
+        perm_out.alloc(nlive * sizeof(uint32_t), false);
+        iota_kernel<<<fill_grid(ctx, nlive), 256, 0, ctx.stream>>>(perm_in.as<uint32_t>(), nlive);
+        SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, word_in.as<unsigned long long>(), word_out.as<unsigned long long>(),
+                                                       perm_in.as<uint32_t>(), perm_out.as<uint32_t>(), (long long)nlive, 0, 63, ctx.stream));
+        d_temp.alloc(temp_bytes, false);
+        for (int w = words - 1; w >= 0; --w) {
+            const int bases = std::min(21, key_len - 21 * w);
+            gather_word_kernel<<<fill_grid(ctx, nlive), 256, 0, ctx.stream>>>(d_keys.as<unsigned long long>(), perm_in.as<uint32_t>(), nlive, words, w,
+                                                                            word_in.as<unsigned long long>());
+            SCG_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(d_temp.ptr, temp_bytes, word_in.as<unsigned long long>(), word_out.as<unsigned long long>(),
+                                                           perm_in.as<uint32_t>(), perm_out.as<uint32_t>(), (long long)nlive, 0, 3 * bases,
+                                                           ctx.stream));
+            std::swap(perm_in, perm_out);
+        }
+        gather_rows_kernel<<<fill_grid(ctx, nlive), 256, 0, ctx.stream>>>(d_keys.as<unsigned long long>(), d_counts.as<uint32_t>(), perm_in.as<uint32_t>(),
+                                                                        nlive, words, out.keys.as<unsigned long long>(), out.counts.as<uint32_t>());
+        SCG_CUDA_CHECK(cudaGetLastError());
+        ctx.launches += 3 + 2 * words;
+    } else if (wide) {
         const int shift1 = 64 - 3 * (key_len - 21);
         compact128_kernel<<<fill_grid(ctx, capacity), 256, 0, ctx.stream>>>(slots.as<ulonglong2>(), counts.as<uint32_t>(), capacity, key_len, shift1,
                                                                           d_keys.as<WideKey>(), d_counts.as<uint32_t>(), d_cursor.as<unsigned long long>());
@@ -273,21 +433,15 @@ void CountTable::sorted(Context& ctx, int key_len, SortedTable& out) {
 // ---------------------------------------------------------------------------------------
 // sorted tables: rendering and merging on the device
 // ---------------------------------------------------------------------------------------
-// one row per thread; a wide key (words == 2) renders bases 0..20 from word 0 and the rest from word 1
+// one row per thread; word w renders bases [21w, min(21w + 21, len))
 __global__ void render_barcodes_kernel(const unsigned long long* __restrict__ keys, const uint32_t* __restrict__ counts, size_t n, int len,
                                        int words, char* __restrict__ strings, int32_t* __restrict__ freq) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         const unsigned long long* row = keys + i * (size_t)words;
         char* out = strings + i * (size_t)len;
-        const int len0 = words == 2 ? 21 : len;
-        unsigned long long k = row[0];
-        for (int b = len0 - 1; b >= 0; --b) {
-            out[b] = "ACGNT"[k & 7ull];
-            k >>= 3;
-        }
-        if (words == 2) {
-            k = row[1];
-            for (int b = len - 1; b >= 21; --b) {
+        for (int w = 0; w < words; ++w) {
+            unsigned long long k = row[w];
+            for (int b = min(len, 21 * w + 21) - 1; b >= 21 * w; --b) {
                 out[b] = "ACGNT"[k & 7ull];
                 k >>= 3;
             }
@@ -401,11 +555,47 @@ __global__ void merge_scatter_b_kernel(const K* __restrict__ ak, size_t na, cons
     }
 }
 
+// A row of a long-key sorted table (N >= 3 text-order words), compared word 0 first.
+template <int N>
+struct LongKey {
+    unsigned long long w[N];
+};
+template <int N>
+__device__ __forceinline__ bool operator<(const LongKey<N>& a, const LongKey<N>& b) {
+    for (int i = 0; i < N; ++i) {
+        if (a.w[i] != b.w[i]) return a.w[i] < b.w[i];
+    }
+    return false;
+}
+template <int N>
+__device__ __forceinline__ bool operator==(const LongKey<N>& a, const LongKey<N>& b) {
+    for (int i = 0; i < N; ++i) {
+        if (a.w[i] != b.w[i]) return false;
+    }
+    return true;
+}
+
+// the longest barcode a template holds (MAX_TEMPLATE bases) takes this many words
+constexpr int MAX_TABLE_WORDS = (MAX_TEMPLATE + 20) / 21;
+
+template <int N, class F>
+static void with_long_key(int words, F&& f) {
+    if constexpr (N > MAX_TABLE_WORDS) {
+        throw Error("internal error: sorted table of " + std::to_string(words) + " words per row");
+    } else if (words == N) {
+        f(LongKey<N>{});
+    } else {
+        with_long_key<N + 1>(words, f);
+    }
+}
+
 // f(K{}) with the key type of tables of `words` words per row
 template <class F>
 static void with_key_type(int words, F&& f) {
     if (words == 2) {
         f(WideKey{});
+    } else if (words > 2) {
+        with_long_key<3>(words, f);
     } else {
         f(0ull);
     }
@@ -671,7 +861,7 @@ void count_random_reader(Context& c, FastqReader* reader, const RandomMatcher& m
 
     c.ensure_ready();
     CountTable tab;
-    tab.init(c, wide, wide ? (1u << 20) : (1u << 23));   // 8 M slots (128 MB) to start with: a few million distinct barcodes need no rehash
+    tab.init(c, wide, (wide || m.long_words) ? (1u << 20) : (1u << 23), m.long_words);   // 8 M slots (128 MB) to start with: a few million distinct barcodes need no rehash
     DeviceBuffer d_odd_out, d_odd_count;
     d_odd_count.alloc(sizeof(unsigned long long), true);
     std::map<std::string, int> extra;   // keys of reads that need their raw text
@@ -753,18 +943,14 @@ void count_random_reader(Context& c, FastqReader* reader, const RandomMatcher& m
         SCG_CUDA_CHECK(cudaMemcpyAsync(cnt.data(), sorted.counts.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
         SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
     }
-    // one row of the table as text: bases 0..20 (or all of a narrow key) from word 0, the rest from word 1
+    // one row of the table as text: word w holds bases [21w, min(21w + 21, key_len))
     auto render = [&](const unsigned long long* row, char* out) {
-        const int len0 = words == 2 ? 21 : key_len;
-        unsigned long long k = row[0];
-        for (int b = len0 - 1; b >= 0; --b) {
-            out[b] = "ACGNT"[k & 7ull];
-            k >>= 3;
-        }
-        k = words == 2 ? row[1] : 0ull;
-        for (int b = key_len - 1; b >= len0; --b) {
-            out[b] = "ACGNT"[k & 7ull];
-            k >>= 3;
+        for (int w = 0; w < words; ++w) {
+            unsigned long long k = row[w];
+            for (int b = std::min(key_len, 21 * w + 21) - 1; b >= 21 * w; --b) {
+                out[b] = "ACGNT"[k & 7ull];
+                k >>= 3;
+            }
         }
     };
     std::unique_ptr<scg_result> r(new scg_result);

@@ -782,11 +782,12 @@ static void launch_random_generic(Context& ctx, const ReadsDev& reads, const Ran
     const RandomParams& P = m.params;
     CountTable64 t64 = m.wide ? CountTable64{ nullptr, 0, nullptr } : tab.view64();
     CountTable128 t128 = m.wide ? tab.view128() : CountTable128{ nullptr, nullptr, 0, nullptr };
+    CountTableLong tl{};
     dispatch_cb(P.spec.cbits, [&](auto CB) {
         if (m.key_len <= 32) {
-            random_kernel<decltype(CB)::value, 1><<<grid, 128, 0, stream>>>(reads, P, t64, t128, odd, 0, odd_out, odd_count, out_index, visit);
+            random_kernel<decltype(CB)::value, 1><<<grid, 128, 0, stream>>>(reads, P, t64, t128, tl, odd, 0, odd_out, odd_count, out_index, visit);
         } else {
-            random_kernel<decltype(CB)::value, 2><<<grid, 128, 0, stream>>>(reads, P, t64, t128, odd, 0, odd_out, odd_count, out_index, visit);
+            random_kernel<decltype(CB)::value, 2><<<grid, 128, 0, stream>>>(reads, P, t64, t128, tl, odd, 0, odd_out, odd_count, out_index, visit);
         }
     });
     SCG_CUDA_CHECK(cudaGetLastError());
@@ -794,9 +795,51 @@ static void launch_random_generic(Context& ctx, const ReadsDev& reads, const Ran
     ++ctx.timing.launches;
 }
 
+// Barcodes of 43 bases or more: the generic kernel into the long-key table (libdev.hpp CountTableLong), over slices of at most
+// LONG_SLICE_READS reads, each followed by the kernel that moves its fresh keys from the staging rows into the key store -- so the
+// staging buffer holds one slice (at most 2^21 rows of up to 13 words, 208 MiB) however many reads the batch has.
+static constexpr long long LONG_SLICE_READS = 1ll << 21;
+
+static void launch_random_long(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, CountTable& tab, const uint8_t* odd,
+                               OddOutcome* odd_out, unsigned long long* odd_count, int32_t* out_index, cudaStream_t stream) {
+    const RandomParams& P = m.params;
+    const CountTable64 t64{ nullptr, 0, nullptr };
+    const CountTable128 t128{ nullptr, nullptr, 0, nullptr };
+    for (long long first = 0; first < reads.n; first += LONG_SLICE_READS) {
+        // a slice starts on a tile boundary (LONG_SLICE_READS is a multiple of TILE)
+        ReadsDev slice = reads;
+        slice.n = std::min(LONG_SLICE_READS, reads.n - first);
+        slice.data = reads.data + (size_t)(first / TILE) * tile_words(reads.W);
+        if (reads.lens) slice.lens = reads.lens + first;
+        const CountTableLong tl = tab.view_long((size_t)slice.n);
+        const uint8_t* slice_odd = odd ? odd + first : nullptr;
+        int32_t* slice_index = out_index ? out_index + first : nullptr;
+        const int grid = ctx.grid_for((slice.n + TILE - 1) / TILE);
+        dispatch_cb(P.spec.cbits, [&](auto CB) {
+            if (m.key_len <= 64) {
+                random_kernel<decltype(CB)::value, 2><<<grid, 128, 0, stream>>>(slice, P, t64, t128, tl, slice_odd, first, odd_out, odd_count, slice_index,
+                                                                                ReadList{ nullptr, nullptr });
+            } else {
+                random_kernel<decltype(CB)::value, 8><<<grid, 128, 0, stream>>>(slice, P, t64, t128, tl, slice_odd, first, odd_out, odd_count, slice_index,
+                                                                                ReadList{ nullptr, nullptr });
+            }
+        });
+        SCG_CUDA_CHECK(cudaGetLastError());
+        ++ctx.launches;
+        ++ctx.timing.launches;
+        tab.promote_fresh(ctx, stream);
+    }
+}
+
 void launch_random(Context& ctx, const ReadsDev& reads, const RandomMatcher& m, CountTable& tab, const uint8_t* odd, OddOutcome* odd_out,
                    unsigned long long* odd_count, int32_t* out_index, cudaStream_t stream) {
     if (reads.n <= 0) return;
+    if (m.long_words) {
+        launch_random_long(ctx, reads, m, tab, odd, odd_out, odd_count, out_index, stream);
+        ctx.kernel_note = "generic random_kernel into the long-key count table (barcodes of " + std::to_string(m.key_len) +
+                          " bases: staged keys, tag claims, promote_fresh_kernel)";
+        return;
+    }
     const long long ntiles = (reads.n + TILE - 1) / TILE;
     std::string why;
     const JitModule* mod = nullptr;
@@ -1049,7 +1092,7 @@ int scg_random_plan_create(scg_ctx* ctx, const char* constant, int strand, int m
         // sized once for the distinct barcodes the caller expects (load factor <= 1/2; a table twice the size keeps more barcodes
         // inside their home sector but measured slower: its footprint costs more than the displaced keys do); 0 = grow as the
         // reference's map does
-        plan->table.init(c, plan->random->wide, expected_distinct > 0 ? (size_t)(2 * expected_distinct) : (size_t)1 << 20);
+        plan->table.init(c, plan->random->wide, expected_distinct > 0 ? (size_t)(2 * expected_distinct) : (size_t)1 << 20, plan->random->long_words);
         plan->table.fixed = expected_distinct > 0;
         SCG_CUDA_CHECK(cudaStreamSynchronize(c.stream));
         *out = plan.release();
@@ -1123,6 +1166,8 @@ int scg_plan_sorted_table(scg_plan* plan, scg_table** out) {
         if (plan->kind == scg_plan::COMBO) {
             plan->tally.sorted(c, t->table);
         } else if (plan->kind == scg_plan::RANDOM) {
+            // what this interface hands out it must be able to take back (scg_table_from_device: key lengths 0..42)
+            if (plan->random->key_len > 42) throw Error("sorted tables hold random barcodes of at most 42 bases");
             plan->table.sorted(c, plan->random->key_len, t->table);
         } else {
             throw Error("only combinatorial and random-barcode plans hold a table");
