@@ -18,13 +18,10 @@
 // < 2^-10).  Text is written to global memory (the FASTQ reader's ring), source bytes of a match are read back from there.
 // A second kernel checks the members' CRC-32 (gzip trailer), one warp per member, 2 KiB per lane, slice-by-4 tables in shared
 // memory, the lanes' partial CRCs combined with the "2 KiB of zeros" operator.
-// A second route (SCG_INFLATE_ROUTE=split, measured and not the default: DESIGN.md 5.4) decodes with one LANE per member into
-// symbols in global memory (decode_tokens_kernel) and assembles the text with one warp per member (place_tokens_kernel).
 #include "inflate.cuh"
 
 #include <algorithm>
 #include <cstdlib>
-#include <cstring>
 
 namespace scg {
 
@@ -89,22 +86,21 @@ __device__ __forceinline__ uint32_t dist_entry(int sym, int len) {
 __device__ __forceinline__ uint32_t clen_entry(int sym, int len) { return ((uint32_t)sym << 6) | (uint32_t)len; }
 
 // Builds the lookup table of a canonical Huffman code from the code lengths lens[0 .. n).  KIND 0 literal/length, 1 distance,
-// 2 code lengths.  All GL lanes of the group take part (gm = their mask, gl = this lane's place among them).  false =
-// over-subscribed set of lengths.
-template <int KIND, int TBITS, int GL>
+// 2 code lengths.  All lanes of the warp take part.  false = over-subscribed set of lengths.
+template <int KIND, int TBITS>
 __device__ bool build_table(const uint8_t* lens, int n, Entry* table, uint16_t* sorted, uint32_t* count, uint32_t* next, uint32_t* offs,
-                            uint32_t gm, int gl) {
+                            int lane) {
     const uint32_t below = (1u << (threadIdx.x & 31)) - 1u;   // the lanes in front of this one
-    for (int i = gl; i < (1 << TBITS); i += GL) table[i] = (Entry)E_INVALID;
-    for (int i = gl; i < 16; i += GL) count[i] = 0;
-    __syncwarp(gm);
-    for (int s = gl; s < n; s += GL) {
+    for (int i = lane; i < (1 << TBITS); i += 32) table[i] = (Entry)E_INVALID;
+    for (int i = lane; i < 16; i += 32) count[i] = 0;
+    __syncwarp();
+    for (int s = lane; s < n; s += 32) {
         const int l = lens[s];
         if (l) atomicAdd(&count[l], 1u);
     }
-    __syncwarp(gm);
+    __syncwarp();
     bool ok = true;
-    if (gl == 0) {
+    if (lane == 0) {
         uint32_t code = 0, off = 0;
         int left = 1;
         for (int l = 1; l <= 15; ++l) {
@@ -116,13 +112,13 @@ __device__ bool build_table(const uint8_t* lens, int n, Entry* table, uint16_t* 
             off += count[l];
         }
     }
-    ok = __shfl_sync(gm, ok ? 1 : 0, 0, GL) != 0;
+    ok = __shfl_sync(FULL, ok ? 1 : 0, 0) != 0;
     if (!ok) return false;
-    __syncwarp(gm);
-    for (int base = 0; base < n; base += GL) {
-        const int s = base + gl;
+    __syncwarp();
+    for (int base = 0; base < n; base += 32) {
+        const int s = base + lane;
         const int l = s < n ? lens[s] : 0;
-        const uint32_t peers = __match_any_sync(gm, l);
+        const uint32_t peers = __match_any_sync(FULL, l);
         const int rank = __popc(peers & below);
         if (l) {
             const uint32_t code = next[l] + (uint32_t)rank;
@@ -135,12 +131,12 @@ __device__ bool build_table(const uint8_t* lens, int n, Entry* table, uint16_t* 
                 table[r & ((1u << TBITS) - 1u)] = (Entry)E_LONG;
             }
         }
-        __syncwarp(gm);
+        __syncwarp();
         if (l && rank == 0) {
             next[l] += (uint32_t)__popc(peers);
             offs[l] += (uint32_t)__popc(peers);
         }
-        __syncwarp(gm);
+        __syncwarp();
     }
     return true;
 }
@@ -165,36 +161,33 @@ __device__ __forceinline__ bool slow_symbol(unsigned long long bits, const uint3
     return false;
 }
 
-// The compressed stream as seen by the group: a window of 64 bits of the stream that stays put between refills, and the
+// The compressed stream as seen by the warp: a window of 64 bits of the stream that stays put between refills, and the
 // number of its bits already consumed -- taking bits moves the position (one add), looking at bits is one 64-bit shift.  The
-// window is refilled, 32 bits at a time, from two register-resident lines of GL words.
-template <int GL>
+// window is refilled, 32 bits at a time, from two register-resident lines of 32 words.
 struct BitReader {
     const uint32_t* words;      // 4-byte aligned base of the stream
     uint32_t line_cur, line_next;
-    uint32_t widx;              // words taken into the window so far (uniform in the group)
+    uint32_t widx;              // words taken into the window so far (uniform in the warp)
     unsigned long long bits;    // stream bits [32 * (widx - 2), 32 * widx)
     int bp;                     // bits of the window consumed
-    uint32_t gm;
-    int gl;
+    int lane;
 
-    __device__ __forceinline__ void open(const uint8_t* comp, size_t byte_off, uint32_t gm_, int gl_) {
-        gm = gm_;
-        gl = gl_;
+    __device__ __forceinline__ void open(const uint8_t* comp, size_t byte_off, int lane_) {
+        lane = lane_;
         words = reinterpret_cast<const uint32_t*>(comp + (byte_off & ~(size_t)3));
-        line_cur = words[gl];
-        line_next = words[GL + gl];
+        line_cur = words[lane];
+        line_next = words[32 + lane];
         widx = 0;
         const uint32_t lo = next_word();
         bits = (unsigned long long)lo | ((unsigned long long)next_word() << 32);
         bp = (int)(byte_off & 3) * 8;
     }
     __device__ __forceinline__ uint32_t next_word() {
-        const uint32_t w = __shfl_sync(gm, line_cur, (int)(widx & (uint32_t)(GL - 1)), GL);
+        const uint32_t w = __shfl_sync(FULL, line_cur, (int)(widx & 31u));
         ++widx;
-        if ((widx & (uint32_t)(GL - 1)) == 0) {
+        if ((widx & 31u) == 0) {
             line_cur = line_next;
-            line_next = words[widx + GL + gl];
+            line_next = words[widx + 32 + lane];
         }
         return w;
     }
@@ -224,80 +217,58 @@ struct BitReader {
 // A match of the batch, copied into the stage: byte j comes from batch-relative position off - dist + j (the repeating
 // pattern of the last `dist` bytes when the match overlaps itself); positions before the batch are text already in global
 // memory (`done` = the batch's first byte there), the others are bytes of the stage written by earlier symbols.
-template <int GL>
-__device__ __forceinline__ void copy_match(uint8_t* stage, const uint8_t* done, uint32_t off, uint32_t len, uint32_t dist, int gl) {
-    for (uint32_t j = gl; j < len; j += GL) {
+__device__ __forceinline__ void copy_match(uint8_t* stage, const uint8_t* done, uint32_t off, uint32_t len, uint32_t dist, int lane) {
+    for (uint32_t j = lane; j < len; j += 32) {
         const int src = (int)off - (int)dist + (int)(dist >= len ? j : j % dist);
         stage[off + j] = src < 0 ? done[src] : stage[src];
     }
 }
 
 // The text of a batch of nsym symbols (A.syms, `total` bytes of text in all) assembled in shared memory and written to
-// out[pos, pos + total).  All GL lanes of the group take part; false = a symbol reaches before the start of the text or
-// the batch beyond its end.
-template <int GL>
-__device__ __forceinline__ bool put_batch(BatchArea& A, int nsym, uint32_t staged, uint8_t* out, uint32_t pos, uint32_t out_len, uint32_t gm, int lane) {
-    constexpr int SPL = 32 / GL;      // symbols of a batch per lane
+// out[pos, pos + total).  All lanes of the warp take part; false = a symbol reaches before the start of the text or the
+// batch beyond its end.
+__device__ __forceinline__ bool put_batch(BatchArea& A, int nsym, uint32_t staged, uint8_t* out, uint32_t pos, uint32_t out_len, int lane) {
     constexpr uint32_t SHORT_MATCH = 12;
-    __syncwarp(gm);
-    // ---- where the batch's symbols go: lane l looks after symbols [l * SPL, (l + 1) * SPL) ----
-    uint32_t my[SPL], mylen[SPL], off[SPL];
-    uint32_t mine = 0;
+    __syncwarp();
+    // ---- where the batch's symbols go: lane l looks after symbol l ----
+    const uint32_t my = lane < nsym ? A.syms[lane] : 0u;
+    const uint32_t mylen = (my >> 16) & 0x1FFu;
+    uint32_t incl = mylen;
 #pragma unroll
-    for (int j = 0; j < SPL; ++j) {
-        const int k = lane * SPL + j;
-        my[j] = k < nsym ? A.syms[k] : 0u;
-        mylen[j] = (my[j] >> 16) & 0x1FFu;
-        off[j] = mine;
-        mine += mylen[j];
-    }
-    uint32_t incl = mine;
-#pragma unroll
-    for (int d = 1; d < GL; d <<= 1) {
-        const uint32_t v = __shfl_up_sync(gm, incl, d, GL);
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t v = __shfl_up_sync(FULL, incl, d);
         if (lane >= d) incl += v;
     }
     const uint32_t total = staged;
-    bool too_far = false;
-    uint32_t long_bits = 0, dep_bits = 0;   // this lane's symbols among the batch's 32, by what copies them
-    bool indep_short[SPL];
-#pragma unroll
-    for (int j = 0; j < SPL; ++j) {
-        off[j] += incl - mine;   // relative to the batch's first byte
-        A.sym_off[lane * SPL + j] = off[j];
-        const bool is_match = mylen[j] != 0 && !(my[j] >> 31);
-        const uint32_t dist = my[j] & 0xFFFFu;
-        too_far |= is_match && dist > pos + off[j];
-        // matches whose source ends before the batch begins: no ordering among them, their loads overlap
-        const bool indep = is_match && off[j] + mylen[j] <= dist;
-        indep_short[j] = indep && mylen[j] <= SHORT_MATCH;
-        if (indep && mylen[j] > SHORT_MATCH) long_bits |= 1u << (lane * SPL + j);
-        if (is_match && !indep) dep_bits |= 1u << (lane * SPL + j);
-    }
-    if (pos + total > out_len || __any_sync(gm, too_far)) {
+    const uint32_t off = incl - mylen;   // relative to the batch's first byte
+    A.sym_off[lane] = off;
+    const bool is_match = mylen != 0 && !(my >> 31);
+    const uint32_t dist = my & 0xFFFFu;
+    const bool too_far = is_match && dist > pos + off;
+    // matches whose source ends before the batch begins: no ordering among them, their loads overlap
+    const bool indep = is_match && off + mylen <= dist;
+    const bool indep_short = indep && mylen <= SHORT_MATCH;
+    // this lane's symbol among the batch's 32, by what copies it
+    const uint32_t long_bits = indep && mylen > SHORT_MATCH ? 1u << lane : 0u;
+    const uint32_t dep_bits = is_match && !indep ? 1u << lane : 0u;
+    if (pos + total > out_len || __any_sync(FULL, too_far)) {
         return false;
     }
     // the stage mirrors the alignment of the text in global memory, so that it can be flushed as aligned words
     uint8_t* const done = out + pos;
     const uint32_t skew = (uint32_t)(reinterpret_cast<size_t>(done) & 3);
     uint8_t* const stage = reinterpret_cast<uint8_t*>(A.stage) + skew;
-#pragma unroll
-    for (int j = 0; j < SPL; ++j) {
-        if (my[j] >> 31) stage[off[j]] = (uint8_t)my[j];
-    }
+    if (my >> 31) stage[off] = (uint8_t)my;
     // Short independent matches (the rule for the bases of a FASTQ record) are copied by the lanes that hold them, all
     // at once: the warp runs as many byte steps as the longest of them has bytes, instead of a round per match.
-#pragma unroll
-    for (int j = 0; j < SPL; ++j) {
-        if (indep_short[j]) {
-            const uint8_t* src = done + ((int)off[j] - (int)(my[j] & 0xFFFFu));
-            for (uint32_t i = 0; i < mylen[j]; ++i) stage[off[j] + i] = src[i];
-        }
+    if (indep_short) {
+        const uint8_t* src = done + ((int)off - (int)dist);
+        for (uint32_t i = 0; i < mylen; ++i) stage[off + i] = src[i];
     }
-    __syncwarp(gm);   // A.sym_off is read below
-    // the longer ones by all lanes of the group together, four matches at a time: a warp issues in order, so the
-    // loads of four matches go out before the first store waits
-    uint32_t todo = __reduce_or_sync(gm, long_bits);
+    __syncwarp();   // A.sym_off is read below
+    // the longer ones by all lanes together, four matches at a time: a warp issues in order, so the loads of four
+    // matches go out before the first store waits
+    uint32_t todo = __reduce_or_sync(FULL, long_bits);
     while (todo) {
         uint32_t sy[4], o[4];
 #pragma unroll
@@ -324,50 +295,44 @@ __device__ __forceinline__ bool put_batch(BatchArea& A, int nsym, uint32_t stage
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             const uint32_t len = (sy[u] >> 16) & 0x1FFu;
-            for (uint32_t j = lane + GL; j < len; j += GL) stage[o[u] + j] = done[(int)o[u] - (int)(sy[u] & 0xFFFFu) + (int)j];
+            for (uint32_t j = lane + 32; j < len; j += 32) stage[o[u] + j] = done[(int)o[u] - (int)(sy[u] & 0xFFFFu) + (int)j];
         }
     }
     // the others read bytes of this batch: in order, each after what precedes it has landed in the stage
-    todo = __reduce_or_sync(gm, dep_bits);
+    todo = __reduce_or_sync(FULL, dep_bits);
     while (todo) {
-        __syncwarp(gm);
+        __syncwarp();
         const int k = __ffs(todo) - 1;
         todo &= todo - 1;
         const uint32_t sy = A.syms[k], o = A.sym_off[k];
-        copy_match<GL>(stage, done, o, (sy >> 16) & 0x1FFu, sy & 0xFFFFu, lane);
+        copy_match(stage, done, o, (sy >> 16) & 0x1FFu, sy & 0xFFFFu, lane);
     }
-    __syncwarp(gm);
+    __syncwarp();
     // ---- the finished batch goes out: whole aligned words, the ragged ends byte by byte ----
     {
         const uint32_t span = skew + total;                 // bytes of the stage in use, from its aligned base
         const uint32_t first_word = skew ? 1u : 0u;         // word 0 is partial when the text does not start aligned
         const uint32_t full_words = span / 4;               // words [first_word, full_words) are complete
         uint32_t* gw = reinterpret_cast<uint32_t*>(done - skew);
-        for (uint32_t w = first_word + lane; w < full_words; w += GL) gw[w] = A.stage[w];
+        for (uint32_t w = first_word + lane; w < full_words; w += 32) gw[w] = A.stage[w];
         const uint8_t* sb = reinterpret_cast<const uint8_t*>(A.stage);
         uint8_t* gb = done - skew;
         if (skew && (uint32_t)lane >= skew && (uint32_t)lane < min(4u, span)) gb[lane] = sb[lane];
         const uint32_t tail = full_words * 4;               // bytes [tail, span) of a last partial word
         if (full_words >= first_word && tail + lane < span && tail + lane >= skew) gb[tail + lane] = sb[tail + lane];
     }
-    __syncwarp(gm);
+    __syncwarp();
     return true;
 }
 
-// GL lanes per member: 32 = one warp per member (what runs); 8 = four members per warp (an experiment, see launch_inflate).
-// WARPS warps per block.
-template <int GL, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __restrict__ comp, const InflateMember* __restrict__ members, int n,
-                                                             uint8_t* out_base, uint32_t* __restrict__ errors) {
-    constexpr int GROUPS = 32 / GL;   // members per warp
-    __shared__ WarpTables tables[WARPS * GROUPS];
-    const int lane32 = threadIdx.x & 31;
-    const int lane = lane32 % GL;                  // this lane's place in its group
-    const int group = lane32 / GL;
-    const uint32_t gm = GL == 32 ? 0xFFFFFFFFu : (((1u << (GL & 31)) - 1u) << (group * GL));
-    WarpTables& T = tables[(threadIdx.x >> 5) * GROUPS + group];
-    const int first_member = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * GROUPS + group;
-    const int member_stride = (int)((gridDim.x * blockDim.x) >> 5) * GROUPS;
+// one warp per member, INFL_WARPS warps per block
+__global__ void __launch_bounds__(INFL_WARPS * 32) inflate_kernel(const uint8_t* __restrict__ comp, const InflateMember* __restrict__ members, int n,
+                                                                  uint8_t* out_base, uint32_t* __restrict__ errors) {
+    __shared__ WarpTables tables[INFL_WARPS];
+    const int lane = threadIdx.x & 31;
+    WarpTables& T = tables[threadIdx.x >> 5];
+    const int first_member = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    const int member_stride = (int)((gridDim.x * blockDim.x) >> 5);
 
     for (int mi = first_member; mi < n; mi += member_stride) {
         const InflateMember M = members[mi];
@@ -375,8 +340,8 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
         uint32_t pos = 0;
         bool bad = false;
         if (M.out_len == 0 && M.in_len <= 2) continue;   // the empty member that closes a BGZF file
-        BitReader<GL> br;
-        br.open(comp, M.in_off, gm, lane);
+        BitReader br;
+        br.open(comp, M.in_off, lane);
         bool last = false;
         while (!last && !bad) {
             // a block header beyond the member's bytes: a damaged stream running away (it must not leave the image)
@@ -400,10 +365,10 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                     break;
                 }
                 const size_t from = (size_t)(reinterpret_cast<const uint8_t*>(br.words) - comp) + br.byte_pos();
-                for (uint32_t j = lane; j < len; j += GL) out[pos + j] = comp[from + j];
+                for (uint32_t j = lane; j < len; j += 32) out[pos + j] = comp[from + j];
                 pos += len;
-                __syncwarp(gm);
-                br.open(comp, from + len, gm, lane);
+                __syncwarp();
+                br.open(comp, from + len, lane);
                 continue;
             }
             if (type == 3) {
@@ -413,8 +378,8 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
             int nlit = 288, ndist = 30;
             if (type == 1) {
                 // ---- fixed codes (RFC 1951 3.2.6) ----
-                for (int s = lane; s < 288; s += GL) T.lens[s] = s < 144 ? 8 : (s < 256 ? 9 : (s < 280 ? 7 : 8));
-                for (int s = lane; s < 30; s += GL) T.lens[288 + s] = 5;
+                for (int s = lane; s < 288; s += 32) T.lens[s] = s < 144 ? 8 : (s < 256 ? 9 : (s < 280 ? 7 : 8));
+                for (int s = lane; s < 30; s += 32) T.lens[288 + s] = 5;
             } else {
                 // ---- dynamic codes: the code-length code first, then the two alphabets' lengths through it ----
                 br.refill();
@@ -425,19 +390,19 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                     bad = true;
                     break;
                 }
-                for (int s = lane; s < 19; s += GL) T.lens[320 + s] = 0;
-                __syncwarp(gm);
+                for (int s = lane; s < 19; s += 32) T.lens[320 + s] = 0;
+                __syncwarp();
                 for (int k = 0; k < nclen; ++k) {
                     br.refill();
                     const uint32_t v = br.take(3);
                     if (lane == 0) T.lens[320 + c_clen_order[k]] = (uint8_t)v;
                 }
-                __syncwarp(gm);
-                if (!build_table<2, 7, GL>(T.lens + 320, 19, T.dist, T.dist_sorted, T.dist_count, T.next, T.offs, gm, lane)) {
+                __syncwarp();
+                if (!build_table<2, 7>(T.lens + 320, 19, T.dist, T.dist_sorted, T.dist_count, T.next, T.offs, lane)) {
                     bad = true;
                     break;
                 }
-                __syncwarp(gm);
+                __syncwarp();
                 int i = 0;
                 uint32_t prev = 0;
                 while (i < nlit + ndist) {
@@ -469,7 +434,7 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                         break;
                     }
                     // lengths of the distance alphabet are kept from offset 288 on
-                    for (uint32_t k = lane; k < rep; k += GL) {
+                    for (uint32_t k = lane; k < rep; k += 32) {
                         const int at = i + (int)k;
                         T.lens[at < nlit ? at : 288 + (at - nlit)] = (uint8_t)val;
                     }
@@ -477,19 +442,19 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                     prev = val;
                 }
                 if (bad) break;
-                __syncwarp(gm);
+                __syncwarp();
                 if (T.lens[256] == 0) {   // no end-of-block code
                     bad = true;
                     break;
                 }
             }
-            __syncwarp(gm);
-            if (!build_table<0, LIT_BITS, GL>(T.lens, nlit, T.lit, T.lit_sorted, T.lit_count, T.next, T.offs, gm, lane) ||
-                !build_table<1, DIST_BITS, GL>(T.lens + 288, ndist, T.dist, T.dist_sorted, T.dist_count, T.next, T.offs, gm, lane)) {
+            __syncwarp();
+            if (!build_table<0, LIT_BITS>(T.lens, nlit, T.lit, T.lit_sorted, T.lit_count, T.next, T.offs, lane) ||
+                !build_table<1, DIST_BITS>(T.lens + 288, ndist, T.dist, T.dist_sorted, T.dist_count, T.next, T.offs, lane)) {
                 bad = true;
                 break;
             }
-            __syncwarp(gm);
+            __syncwarp();
 
             // ---- the block's symbols, a batch at a time ----
             bool end_of_block = false;
@@ -502,7 +467,7 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                 }
                 // symbols are parked in shared memory: literal = 1 << 31 | 1 << 16 | byte; match = len << 16 | dist
                 int nsym = 0;
-                uint32_t staged = 0;   // bytes the batch produces so far (uniform in the group)
+                uint32_t staged = 0;   // bytes the batch produces so far (uniform in the warp)
 #pragma unroll 1
                 for (; nsym < 32 && staged <= STAGE_BYTES - 258; ++nsym) {
                     br.refill();
@@ -549,10 +514,10 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
                         sym = (len << 16) | dist;
                         staged += len;
                     }
-                    T.batch.syms[nsym] = sym;   // every lane of the group stores the same word
+                    T.batch.syms[nsym] = sym;   // every lane stores the same word
                 }
                 if (bad) break;
-                if (!put_batch<GL>(T.batch, nsym, staged, out, pos, M.out_len, gm, lane)) {
+                if (!put_batch(T.batch, nsym, staged, out, pos, M.out_len, lane)) {
                     bad = true;
                     break;
                 }
@@ -564,338 +529,6 @@ __global__ void __launch_bounds__(WARPS * 32) inflate_kernel(const uint8_t* __re
             const size_t end_bit = (size_t)(reinterpret_cast<const uint8_t*>(br.words) - comp) * 8 + br.bit_pos();
             bad = pos != M.out_len || end_bit > ((size_t)M.in_off + M.in_len) * 8;
         }
-        if (bad && lane == 0) atomicOr(errors, 1u);
-        __syncwarp(gm);
-    }
-}
-
-// ---- the two-kernel route: one LANE decodes a member into symbols, one WARP turns a member's symbols into text ------------------
-// Huffman decoding gives a warp nothing to share: in inflate_kernel all 32 lanes run the same 80 instructions per symbol.  Here
-// every lane decodes a member of its own (its code tables in shared memory, interleaved by lane so that 32 different lookups hit
-// 32 different banks; 10-bit literal/length and 7-bit distance tables, 2304 bytes per lane, three warps per SM), and leaves the
-// member's symbols -- the words put_batch takes -- in global memory: symbol i of the member whose text starts at out_off is
-// tokens[out_off + i] (a symbol stands for at least one byte of text, so a member's symbols fit where four times its text would).
-// place_tokens_kernel then assembles the text, a warp per member, 32 symbols per round.
-constexpr int DEC_DIST_BITS = 7;
-constexpr int dec_smem_bytes(int lit_bits) { return ((1 << lit_bits) + (1 << DEC_DIST_BITS)) * 2 * 32; }
-
-// entry i of this lane's table: 16-bit entries, two per word, the words of the 32 lanes side by side
-struct LaneTable {
-    uint16_t* base;   // this lane's half-word 0
-    __device__ __forceinline__ uint16_t* at(uint32_t i) const { return base + ((i >> 1) << 6) + (i & 1u); }
-    __device__ __forceinline__ uint32_t get(uint32_t i) const { return *at(i); }
-    __device__ __forceinline__ void set(uint32_t i, uint32_t e) const { *at(i) = (uint16_t)e; }
-};
-
-// canonical code of the lengths lens[0 .. n) into a lane's table; count / sorted are kept for the codes longer than the table
-template <int KIND, int TBITS>
-__device__ bool lane_build_table(const uint8_t* lens, int n, const LaneTable& table, uint32_t* count, uint16_t* sorted) {
-    uint32_t next[16], offs[16];
-    for (uint32_t i = 0; i < (1u << TBITS); ++i) table.set(i, E_INVALID);
-    for (int l = 0; l < 16; ++l) count[l] = 0;
-    for (int s = 0; s < n; ++s) ++count[lens[s]];
-    count[0] = 0;
-    uint32_t code = 0, off = 0;
-    int left = 1;
-    bool ok = true;
-    for (int l = 1; l <= 15; ++l) {
-        next[l] = code;
-        offs[l] = off;
-        left = (left << 1) - (int)count[l];
-        if (left < 0) ok = false;
-        code = (code + count[l]) << 1;
-        off += count[l];
-    }
-    if (!ok) return false;
-    for (int s = 0; s < n; ++s) {
-        const int l = lens[s];
-        if (!l) continue;
-        const uint32_t c = next[l]++;
-        sorted[offs[l]++] = (uint16_t)s;
-        const uint32_t r = __brev(c) >> (32 - l);
-        if (l <= TBITS) {
-            const uint32_t e = KIND == 0 ? lit_entry(s, l) : (KIND == 1 ? dist_entry(s, l) : clen_entry(s, l));
-            for (uint32_t k = r; k < (1u << TBITS); k += (1u << l)) table.set(k, e);
-        } else {
-            table.set(r & ((1u << TBITS) - 1u), E_LONG);
-        }
-    }
-    return true;
-}
-
-template <int DEC_LIT_BITS>
-__global__ void __launch_bounds__(32) decode_tokens_kernel(const uint8_t* __restrict__ comp, const InflateMember* __restrict__ members, int n,
-                                                           uint32_t* __restrict__ tokens, uint32_t* __restrict__ ntok, uint32_t* __restrict__ errors) {
-    extern __shared__ uint32_t dec_smem[];
-    const int lane = threadIdx.x;
-    const LaneTable lit{ reinterpret_cast<uint16_t*>(dec_smem + lane) };
-    const LaneTable dst{ reinterpret_cast<uint16_t*>(dec_smem + (1 << (DEC_LIT_BITS - 1)) * 32 + lane) };
-    uint8_t lens[288 + 32 + 32];
-    uint16_t lit_sorted[288], dist_sorted[32];
-    uint32_t lit_count[16], dist_count[16];
-
-    for (int mi = (int)blockIdx.x * 32 + lane; mi < n; mi += (int)gridDim.x * 32) {
-        const InflateMember M = members[mi];
-        uint32_t* const tok = tokens + M.out_off;
-        uint32_t nt = 0, pos = 0;
-        bool bad = false;
-        if (M.out_len == 0 && M.in_len <= 2) {   // the empty member that closes a BGZF file
-            ntok[mi] = 0;
-            continue;
-        }
-        // the stream: a window of 64 bits that stays put between refills and the number of its bits consumed (as BitReader)
-        const uint32_t* words = reinterpret_cast<const uint32_t*>(comp + ((size_t)M.in_off & ~(size_t)3));
-        uint32_t wmax = (((uint32_t)M.in_off & 3u) + M.in_len + 3u) / 4u + 2u;   // no word beyond the member's (+ look-ahead)
-        uint32_t wi = 2;
-        unsigned long long bits = (unsigned long long)words[0] | ((unsigned long long)words[1] << 32);
-        uint32_t ahead = words[2];   // the word that enters the window next
-        int bp = (int)(M.in_off & 3u) * 8;
-#define DEC_REFILL()                                                                 \
-    do {                                                                             \
-        if (bp >= 32) {                                                              \
-            if (wi > wmax) bad = true;                                               \
-            bits = (bits >> 32) | ((unsigned long long)ahead << 32);                 \
-            ++wi;                                                                    \
-            ahead = words[bad ? 0 : wi];   /* used at the next refill: its latency is off the decoding chain */ \
-            bp -= 32;                                                                \
-        }                                                                            \
-    } while (0)
-#define DEC_TAKE(v, nb)                                              \
-    do {                                                             \
-        v = (uint32_t)(bits >> bp) & ((1u << (nb)) - 1u);            \
-        bp += (nb);                                                  \
-    } while (0)
-        bool last = false, in_block = false;
-        for (;;) {
-            if (bad) break;
-            if (!in_block) {
-                if (last) break;
-                // ---- block header ----
-                DEC_REFILL();
-                uint32_t v, type;
-                DEC_TAKE(v, 1);
-                last = v != 0;
-                DEC_TAKE(type, 2);
-                if (type == 0) {
-                    // stored: to the byte boundary, LEN, NLEN, LEN raw bytes -- every byte becomes a literal symbol
-                    bp = (bp + 7) & ~7;
-                    DEC_REFILL();
-                    uint32_t len, nlen;
-                    DEC_TAKE(len, 16);
-                    DEC_REFILL();
-                    DEC_TAKE(nlen, 16);
-                    if ((len ^ nlen) != 0xFFFFu || pos + len > M.out_len) {
-                        bad = true;
-                        break;
-                    }
-                    const size_t from = (size_t)(reinterpret_cast<const uint8_t*>(words) - comp) + (size_t)wi * 4 - 8 + (size_t)(bp >> 3);
-                    if (from + len > (size_t)M.in_off + M.in_len) {
-                        bad = true;
-                        break;
-                    }
-                    for (uint32_t j = 0; j < len; ++j) tok[nt + j] = 0x80010000u | comp[from + j];
-                    nt += len;
-                    pos += len;
-                    // the reader again, after the raw bytes
-                    const size_t at = from + len;
-                    words = reinterpret_cast<const uint32_t*>(comp + (at & ~(size_t)3));
-                    wi = 2;
-                    bits = (unsigned long long)words[0] | ((unsigned long long)words[1] << 32);
-                    ahead = words[2];
-                    bp = (int)(at & 3) * 8;
-                    wmax = (uint32_t)(((at & 3) + ((size_t)M.in_off + M.in_len - at) + 3) / 4 + 2);
-                    continue;
-                }
-                if (type == 3) {
-                    bad = true;
-                    break;
-                }
-                int nlit = 288, ndist = 30;
-                if (type == 1) {
-                    for (int s = 0; s < 288; ++s) lens[s] = s < 144 ? 8 : (s < 256 ? 9 : (s < 280 ? 7 : 8));
-                    for (int s = 0; s < 30; ++s) lens[288 + s] = 5;
-                } else {
-                    DEC_REFILL();
-                    uint32_t a, b, c;
-                    DEC_TAKE(a, 5);
-                    DEC_TAKE(b, 5);
-                    DEC_TAKE(c, 4);
-                    nlit = (int)a + 257;
-                    ndist = (int)b + 1;
-                    const int nclen = (int)c + 4;
-                    if (nlit > 286 || ndist > 30) {
-                        bad = true;
-                        break;
-                    }
-                    for (int s = 0; s < 19; ++s) lens[320 + s] = 0;
-                    for (int k = 0; k < nclen; ++k) {
-                        DEC_REFILL();
-                        DEC_TAKE(v, 3);
-                        lens[320 + c_clen_order[k]] = (uint8_t)v;
-                    }
-                    if (!lane_build_table<2, DEC_DIST_BITS>(lens + 320, 19, dst, dist_count, dist_sorted)) {
-                        bad = true;
-                        break;
-                    }
-                    int i = 0;
-                    uint32_t prev = 0;
-                    while (i < nlit + ndist && !bad) {
-                        DEC_REFILL();
-                        const uint32_t e = dst.get((uint32_t)(bits >> bp) & 127u);
-                        if ((e & 0xFu) == 0) {
-                            bad = true;
-                            break;
-                        }
-                        bp += (int)(e & 0xFu);
-                        const uint32_t sym = e >> 6;
-                        uint32_t rep = 1, val = sym;
-                        if (sym == 16) {
-                            if (i == 0) {
-                                bad = true;
-                                break;
-                            }
-                            val = prev;
-                            DEC_TAKE(rep, 2);
-                            rep += 3;
-                        } else if (sym == 17) {
-                            val = 0;
-                            DEC_TAKE(rep, 3);
-                            rep += 3;
-                        } else if (sym == 18) {
-                            val = 0;
-                            DEC_TAKE(rep, 7);
-                            rep += 11;
-                        }
-                        if (i + (int)rep > nlit + ndist) {
-                            bad = true;
-                            break;
-                        }
-                        for (uint32_t k = 0; k < rep; ++k) {
-                            const int at = i + (int)k;
-                            lens[at < nlit ? at : 288 + (at - nlit)] = (uint8_t)val;
-                        }
-                        i += (int)rep;
-                        prev = val;
-                    }
-                    if (bad) break;
-                    if (lens[256] == 0) {   // no end-of-block code
-                        bad = true;
-                        break;
-                    }
-                }
-                if (!lane_build_table<0, DEC_LIT_BITS>(lens, nlit, lit, lit_count, lit_sorted) ||
-                    !lane_build_table<1, DEC_DIST_BITS>(lens + 288, ndist, dst, dist_count, dist_sorted)) {
-                    bad = true;
-                    break;
-                }
-                in_block = true;
-                continue;
-            }
-            // ---- one symbol of the block ----
-            DEC_REFILL();
-            const uint32_t w = (uint32_t)(bits >> bp);
-            uint32_t e = lit.get(w & ((1u << DEC_LIT_BITS) - 1u));
-            if ((e & 0xFu) == 0) {
-                int sym = 256, len = lens[256];
-                if (e == E_LONG) e = slow_symbol(bits >> bp, lit_count, lit_sorted, sym, len) ? lit_entry(sym, len) : E_INVALID;
-                if ((e & 0xFu) == 0) {
-                    if (e == E_EOB) {
-                        bp += len;
-                        in_block = false;
-                        continue;
-                    }
-                    bad = true;
-                    break;
-                }
-            }
-            const uint32_t elen = e & 0xFu;
-            if (!(e & E_MATCH)) {
-                bp += (int)elen;
-                if (pos >= M.out_len) {
-                    bad = true;
-                    break;
-                }
-                tok[nt++] = 0x80010000u | (e >> 8);
-                pos += 1;
-            } else {
-                const uint32_t xl = (e >> 5) & 7u;
-                const uint32_t len = (e >> 8) + 3u + ((w >> elen) & ((1u << xl) - 1u));
-                bp += (int)(elen + xl);
-                DEC_REFILL();
-                const uint32_t w2 = (uint32_t)(bits >> bp);
-                uint32_t d = dst.get(w2 & ((1u << DEC_DIST_BITS) - 1u));
-                if ((d & 0xFu) == 0) {
-                    int dsym = 0, dlen = 0;
-                    if (d == E_LONG) d = slow_symbol(bits >> bp, dist_count, dist_sorted, dsym, dlen) ? dist_entry(dsym, dlen) : E_INVALID;
-                    if ((d & 0xFu) == 0) {
-                        bad = true;
-                        break;
-                    }
-                }
-                const uint32_t dl = d & 0xFu, xd = (d >> 4) & 0xFu;
-                const uint32_t dist = ((d >> 8) << xd) + 1u + ((w2 >> dl) & ((1u << xd) - 1u));
-                bp += (int)(dl + xd);
-                if (pos + len > M.out_len || dist > pos) {
-                    bad = true;
-                    break;
-                }
-                tok[nt++] = (len << 16) | dist;
-                pos += len;
-            }
-        }
-#undef DEC_REFILL
-#undef DEC_TAKE
-        // the stream must end inside the member and produce exactly its text
-        if (!bad) {
-            const size_t end_bit = (size_t)(reinterpret_cast<const uint8_t*>(words) - comp) * 8 + (size_t)wi * 32 - 64 + (size_t)bp;
-            bad = pos != M.out_len || end_bit > ((size_t)M.in_off + M.in_len) * 8;
-        }
-        if (bad) atomicOr(errors, 1u);
-        ntok[mi] = bad ? 0u : nt;
-    }
-}
-
-// a warp per member: 32 symbols per round (fewer when their text would not fit the stage), assembled by put_batch
-__global__ void __launch_bounds__(INFL_WARPS * 32) place_tokens_kernel(const InflateMember* __restrict__ members, int n, const uint32_t* __restrict__ tokens,
-                                                                       const uint32_t* __restrict__ ntok, uint8_t* out_base, uint32_t* __restrict__ errors) {
-    __shared__ BatchArea areas[INFL_WARPS];
-    BatchArea& A = areas[threadIdx.x >> 5];
-    const int lane = threadIdx.x & 31;
-    const int first_member = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    const int member_stride = (int)((gridDim.x * blockDim.x) >> 5);
-    for (int mi = first_member; mi < n; mi += member_stride) {
-        const InflateMember M = members[mi];
-        const uint32_t* tok = tokens + M.out_off;
-        const uint32_t nt = ntok[mi];
-        uint8_t* out = out_base + M.out_off;
-        uint32_t pos = 0, cursor = 0;
-        bool bad = false;
-        while (cursor < nt) {
-            const uint32_t t = cursor + lane < nt ? tok[cursor + lane] : 0u;
-            const uint32_t len = (t >> 16) & 0x1FFu;
-            uint32_t incl = len;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const uint32_t v = __shfl_up_sync(FULL, incl, d);
-                if (lane >= d) incl += v;
-            }
-            // the symbols taken: those that start while the stage could still take a longest match
-            const uint32_t fits = __ballot_sync(FULL, len != 0 && incl - len <= STAGE_BYTES - 258);
-            const int nsym = __popc(fits);   // symbols are taken from the front: the lanes that fit are the first nsym
-            if (nsym == 0) {                 // a zero word among the symbols: not something the decoder writes
-                bad = true;
-                break;
-            }
-            const uint32_t staged = __shfl_sync(FULL, incl, nsym - 1);
-            A.syms[lane] = t;
-            if (!put_batch<32>(A, nsym, staged, out, pos, M.out_len, FULL, lane)) {
-                bad = true;
-                break;
-            }
-            pos += staged;
-            cursor += (uint32_t)nsym;
-        }
-        if (!bad && nt != 0) bad = pos != M.out_len;
         if (bad && lane == 0) atomicOr(errors, 1u);
         __syncwarp();
     }
@@ -1020,57 +653,12 @@ CrcOperator make_crc_operator() {
 
 } // namespace
 
-bool inflate_split_route() {
-    static const bool split = [] {
-        const char* env = std::getenv("SCG_INFLATE_ROUTE");
-        return env && std::strcmp(env, "split") == 0;
-    }();
-    return split;
-}
-
-int launch_inflate(const uint8_t* comp, const InflateMember* members, int n, uint8_t* out, uint32_t* errors, int sm_count, cudaStream_t stream,
-                   uint32_t* scratch, size_t scratch_words, size_t text_bytes) {
+int launch_inflate(const uint8_t* comp, const InflateMember* members, int n, uint8_t* out, uint32_t* errors, int sm_count, cudaStream_t stream) {
     if (n <= 0) return 0;
     static const CrcOperator op = make_crc_operator();
     static const bool check_crc = !std::getenv("SCG_BGZF_NO_CRC");
     const int blocks = std::max(1, std::min((n + INFL_WARPS - 1) / INFL_WARPS, sm_count * 8));
-    if (inflate_split_route() && scratch && scratch_words >= inflate_scratch_words(text_bytes, (size_t)n)) {
-        uint32_t* tokens = scratch;
-        uint32_t* ntok = scratch + text_bytes;
-        static const int lit_bits = [] {
-            const char* env = std::getenv("SCG_INFLATE_LIT_BITS");
-            return env && std::atoi(env) == 10 ? 10 : 9;
-        }();
-        if (lit_bits == 10) {
-            cudaFuncSetAttribute(decode_tokens_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, dec_smem_bytes(10));
-            decode_tokens_kernel<10><<<std::max(1, std::min((n + 31) / 32, sm_count * 3)), 32, dec_smem_bytes(10), stream>>>(comp, members, n, tokens, ntok, errors);
-        } else {
-            cudaFuncSetAttribute(decode_tokens_kernel<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, dec_smem_bytes(9));
-            decode_tokens_kernel<9><<<std::max(1, std::min((n + 31) / 32, sm_count * 5)), 32, dec_smem_bytes(9), stream>>>(comp, members, n, tokens, ntok, errors);
-        }
-        const int pblocks = std::max(1, std::min((n + INFL_WARPS - 1) / INFL_WARPS, sm_count * 16));
-        place_tokens_kernel<<<pblocks, INFL_WARPS * 32, 0, stream>>>(members, n, tokens, ntok, out, errors);
-        if (!check_crc) return 2;
-        crc_kernel<<<blocks, INFL_WARPS * 32, 0, stream>>>(members, n, out, op, errors);
-        return 3;
-    }
-    // SCG_INFLATE_LANES = lanes per member: 32 = one warp per member; 16 / 8 = two / four members per warp, which then share
-    // the (per-lane identical) decoding instructions as long as their streams take the same turns, each member's batch of 32
-    // symbols spread over fewer lanes.  Blocks are sized so that the members' tables fit the 48 KB of static shared memory.
-    static const int lanes = [] {
-        const char* env = std::getenv("SCG_INFLATE_LANES");
-        const int v = env ? std::atoi(env) : 0;
-        return v == 8 || v == 16 ? v : 32;
-    }();
-    if (lanes == 32) {
-        inflate_kernel<32, INFL_WARPS><<<blocks, INFL_WARPS * 32, 0, stream>>>(comp, members, n, out, errors);
-    } else if (lanes == 16) {
-        constexpr int W = 2, per_block = W * 2;
-        inflate_kernel<16, W><<<std::max(1, std::min((n + per_block - 1) / per_block, sm_count * 9)), W * 32, 0, stream>>>(comp, members, n, out, errors);
-    } else {
-        constexpr int W = 1, per_block = W * 4;
-        inflate_kernel<8, W><<<std::max(1, std::min((n + per_block - 1) / per_block, sm_count * 9)), W * 32, 0, stream>>>(comp, members, n, out, errors);
-    }
+    inflate_kernel<<<blocks, INFL_WARPS * 32, 0, stream>>>(comp, members, n, out, errors);
     if (!check_crc) return 1;
     crc_kernel<<<blocks, INFL_WARPS * 32, 0, stream>>>(members, n, out, op, errors);
     return 2;

@@ -22,13 +22,6 @@ struct InflateMember {
 // is OR-ed with 1 when a stream is malformed or does not produce exactly out_len bytes, with 2 when a CRC does not match.  `comp`
 // must be readable for 512 bytes beyond the last member (the readers fetch whole 128-byte lines ahead).  Returns the number of
 // kernels launched.
-// One warp per member decodes and copies.  With SCG_INFLATE_ROUTE=split and `scratch` (device words, at least
-// inflate_scratch_words(text bytes of the n members, n) of them) the work is split in two kernels instead: one LANE per member
-// decodes it into symbols kept in the scratch, one warp per member turns the symbols into text (measured, not the default:
-// DESIGN.md 5.4).
-int launch_inflate(const uint8_t* comp, const InflateMember* members, int n, uint8_t* out, uint32_t* errors, int sm_count, cudaStream_t stream,
-                   uint32_t* scratch = nullptr, size_t scratch_words = 0, size_t text_bytes = 0);
-inline size_t inflate_scratch_words(size_t text_bytes, size_t members) { return text_bytes + members + 64; }
-bool inflate_split_route();   // SCG_INFLATE_ROUTE=split
+int launch_inflate(const uint8_t* comp, const InflateMember* members, int n, uint8_t* out, uint32_t* errors, int sm_count, cudaStream_t stream);
 
 } // namespace scg

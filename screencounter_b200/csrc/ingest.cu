@@ -364,10 +364,8 @@ bool device_inflate_enabled() {
     return !(v && *v && *v != '0');
 }
 
-void IngestBuffers::ensure_bgzf(size_t comp_bytes, size_t nmembers, size_t text_bytes, int slots) {
-    if (inflate_split_route()) symbol_words = std::max(symbol_words, inflate_scratch_words(text_bytes, std::max<size_t>(nmembers, 1)));
+void IngestBuffers::ensure_bgzf(size_t comp_bytes, size_t nmembers, int slots) {
     for (int k = 0; k < slots; ++k) {
-        if (symbol_words) symbols[k].reserve(symbol_words * sizeof(uint32_t));
         comp[k].reserve(comp_bytes + 1024);   // the inflate kernel's readers fetch whole lines ahead
         members[k].reserve(std::max<size_t>(nmembers, 1) * sizeof(InflateMember));
         members_host[k].reserve(std::max<size_t>(nmembers, 1) * sizeof(InflateMember));
@@ -466,7 +464,6 @@ DeviceIngest::DeviceIngest(Context& ctx, const BgzfIndex* image, int nthreads, i
         const BgzfBlock& lastb = bgzf_->blocks[b - 1];
         max_comp_ = std::max(max_comp_, lastb.data + lastb.csize - bgzf_->blocks[first].data);
         max_members_ = std::max(max_members_, b - first);
-        max_text_ = std::max(max_text_, bytes);
     }
     chunk_begin_.push_back(size_);
     chunk_block_.push_back(nb);
@@ -484,7 +481,7 @@ void DeviceIngest::setup(bool source_pinned) {
     if (bgzf_) slots_ = (int)std::max<size_t>(2, std::min<size_t>((size_t)slots_, nchunks() + 1));   // a small file does not need the whole ring
     B.ensure(chunk_, carry_, pinned_source_ ? 0 : (bgzf_ ? max_comp_ : chunk_), slots_);
     if (bgzf_) {
-        B.ensure_bgzf(max_comp_, max_members_, max_text_, slots_);
+        B.ensure_bgzf(max_comp_, max_members_, slots_);
         SCG_CUDA_CHECK(cudaMemsetAsync(B.inflate_errors.ptr, 0, 16, B.copy_stream));
         SCG_CUDA_CHECK(cudaStreamSynchronize(B.copy_stream));   // (the chunks' kernels run on several streams)
     }
@@ -560,10 +557,7 @@ void DeviceIngest::issue_inflate(size_t chunk) {
     SCG_CUDA_CHECK(cudaEventRecord(B.bounced[s], cs));
     B.bounced_valid[s] = true;
     const int launched = launch_inflate(B.comp[s].as<uint8_t>(), B.members[s].as<InflateMember>(), (int)(lb - fb), dst,
-                                        B.inflate_errors.as<uint32_t>(), ctx_.sm_count, cs,
-                                        (!B.symbol_words || chunk < (size_t)env_size("SCG_INFLATE_WARP_FIRST", 2, 0, 1000)) ? nullptr : B.symbols[s].as<uint32_t>(),
-                                        B.symbol_words,
-                                        (size_t)(bgzf_->text_off[lb] - bgzf_->text_off[fb]));
+                                        B.inflate_errors.as<uint32_t>(), ctx_.sm_count, cs);
     SCG_CUDA_CHECK(cudaGetLastError());
     ctx_.launches += launched;
     ctx_.timing.launches += launched;

@@ -97,7 +97,6 @@ private:
     size_t skip_front_ = 0;             // text bytes of the first member that precede the part being read
     size_t max_comp_ = 0;               // most compressed bytes any chunk holds
     size_t max_members_ = 0;
-    size_t max_text_ = 0;       // text bytes of the largest chunk (sizes the symbol scratch of the inflate kernels)
     std::vector<char> block_cache_;     // host-inflated member for raw_read()
     size_t block_cached_ = (size_t)-1;
 
@@ -136,8 +135,6 @@ struct IngestBuffers {
     PinnedBuffer meta;
     // block-gzip input: the compressed members of the chunk in each slot, their table, the inflate kernels' error word
     DeviceBuffer comp[DeviceIngest::kMaxSlots], members[DeviceIngest::kMaxSlots], inflate_errors;
-    DeviceBuffer symbols[DeviceIngest::kMaxSlots];   // the members' decoded symbols, between the two inflate kernels (inflate.cuh)
-    size_t symbol_words = 0;
     PinnedBuffer members_host[DeviceIngest::kMaxSlots];
     cudaStream_t copy_stream = nullptr;                                  // = copy_streams[0]
     cudaStream_t copy_streams[DeviceIngest::kCopyStreams] = {};          // block-gzip chunks take them in turn
@@ -149,7 +146,7 @@ struct IngestBuffers {
     bool bounced_valid[DeviceIngest::kMaxSlots] = {};
     ~IngestBuffers();
     void ensure(size_t chunk, size_t carry, size_t bounce_bytes, int slots);
-    void ensure_bgzf(size_t comp_bytes, size_t nmembers, size_t text_bytes, int slots);
+    void ensure_bgzf(size_t comp_bytes, size_t nmembers, int slots);
 };
 
 // false when the device reader is switched off (environment SCG_HOST_PARSE=1): every input then takes the host parser.

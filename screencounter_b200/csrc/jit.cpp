@@ -216,7 +216,7 @@ std::string SpecSingleConfig::key() const {
     std::ostringstream o;
     o << fbases << '|' << rbases << '|' << T << '|' << fwd << rev << '|' << W << '|' << nb << '|' << cb << '|' << mm << '|' << maxmm << '|' << use_first << '|'
       << fstart << '|' << rstart << '|' << keylen << '|' << dup_first << '|' << ulen << '|' << info << '|' << joint << '|' << has_index << '|' << ibuckets << '|' << ragged
-      << '|' << hist << '|' << pred;
+      << '|' << hist;
     for (uint32_t m : seed_masks) o << '|' << m;
     return o.str();
 }
@@ -414,7 +414,6 @@ cudaKernel_t specialised_single_kernel(const SpecSingleConfig& cfg, int device, 
         << "#define SPEC_IBUCKETS " << cfg.ibuckets << "\n"
         << "#define SPEC_RAGGED " << cfg.ragged << "\n"
         << "#define SPEC_HIST " << cfg.hist << "\n"
-        << "#define SPEC_PRED " << cfg.pred << "\n"
         << "#define SPEC_UWARP " << jit_env_int("SCG_SPEC_UWARP", 0, 0, 1) << "\n"
         << "#define SPEC_SKIP_GENERAL " << (cfg.ulen > 0 ? 1 : 0) << "\n"
         << "#include \"spec_single.cuh\"\n";

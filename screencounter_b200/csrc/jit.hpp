@@ -30,7 +30,6 @@ struct SpecSingleConfig {
     int has_index = 1;            // the per-read index is asked for
     int ibuckets = 0;             // seed buckets with the first candidate inline are there
     int ragged = 0;               // the batch carries per-read lengths (ulen is then the longest read)
-    int pred = 0;                 // memory operations of the settle / probe steps as predicated instructions instead of branches
     int hist = 0;                 // > 0: counters privatised in shared memory, this many (pool size rounded up), flushed at the end
     std::string key() const;
 };

@@ -40,9 +40,7 @@ int scg_bgzf_inflate(scg_ctx* ctx, const void* image, size_t size, char* text, s
             const BgzfBlock& blk = index.blocks[b];
             members[b] = InflateMember{ (uint32_t)blk.data, blk.csize, (uint32_t)index.text_off[b], blk.isize, blk.crc };
         }
-        DeviceBuffer d_comp, d_members, d_out, d_err, d_symbols;
-        const size_t symbol_words = inflate_split_route() ? inflate_scratch_words(index.text_size(), n) : 0;
-        if (symbol_words) d_symbols.alloc(symbol_words * sizeof(uint32_t), false);
+        DeviceBuffer d_comp, d_members, d_out, d_err;
         d_comp.alloc(size + 1024, false);
         d_members.upload(members.data(), n * sizeof(InflateMember), c.stream);
         d_out.alloc(index.text_size() + 256, false);
@@ -53,7 +51,7 @@ int scg_bgzf_inflate(scg_ctx* ctx, const void* image, size_t size, char* text, s
         SCG_CUDA_CHECK(cudaEventCreate(&e1));
         SCG_CUDA_CHECK(cudaEventRecord(e0, c.stream));
         c.launches += launch_inflate(d_comp.as<uint8_t>(), d_members.as<InflateMember>(), (int)n, d_out.as<uint8_t>(), d_err.as<uint32_t>(),
-                                     c.sm_count, c.stream, symbol_words ? d_symbols.as<uint32_t>() : nullptr, symbol_words, index.text_size());
+                                     c.sm_count, c.stream);
         SCG_CUDA_CHECK(cudaGetLastError());
         SCG_CUDA_CHECK(cudaEventRecord(e1, c.stream));
         uint32_t err = 0;

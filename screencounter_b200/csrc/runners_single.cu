@@ -381,7 +381,6 @@ void launch_single(Context& ctx, const ReadsDev& reads, const SingleMatcher& m, 
             // kernel's 8 blocks per SM resident)
             const int hist_max = jit_env_int("SCG_SPEC_HIST_MAX", 1024, 0, 8192);
             if (m.npool > 0 && m.npool <= hist_max) cfg.hist = (m.npool + 31) / 32 * 32;
-            cfg.pred = jit_env_int("SCG_SPEC_PRED", 0, 0, 1);
         }
     }
     std::string why;

@@ -118,9 +118,6 @@
 // > 0: the pool is small enough for the counters to be PRIVATISED IN SHARED MEMORY (one histogram of SPEC_HIST ints per block,
 // shared-memory atomics per matched read, one global atomic per non-zero counter and block at the end) -- the reference's
 // per-thread counter + reduce() of handlers/SingleBarcodeSingleEnd.hpp:93-104,119-125.  Uniform-length kernel only.
-#ifndef SPEC_PRED
-#define SPEC_PRED 0
-#endif
 #ifndef SPEC_UWARP
 #define SPEC_UWARP 0
 #endif
@@ -219,20 +216,6 @@ __device__ __forceinline__ void count_hit(int32_t* __restrict__ counts, uint32_t
 #else
     atomicAdd(counts + index, 1);
 #endif
-}
-
-// Memory operations under a predicate instead of a branch (SPEC_PRED): a conditional block costs BSSY + BRA + BSYNC and makes the
-// compiler re-materialise the memory descriptor inside it; one predicated instruction does not.
-__device__ __forceinline__ void pred_red_add1(int32_t* addr, bool p) {
-    asm volatile("{ .reg .pred q; setp.ne.b32 q, %0, 0; @q red.global.add.s32 [%1], 1; }" ::"r"((int)p), "l"(addr) : "memory");
-}
-__device__ __forceinline__ void pred_stcs(int32_t* addr, int v, bool p) {
-    asm volatile("{ .reg .pred q; setp.ne.b32 q, %0, 0; @q st.global.cs.s32 [%1], %2; }" ::"r"((int)p), "l"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void pred_ldcg(uint4& v, const uint4* addr, bool p) {
-    asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; @q ld.global.cg.v4.u32 {%0, %1, %2, %3}, [%5]; }"
-                 : "+r"(v.x), "+r"(v.y), "+r"(v.z), "+r"(v.w)
-                 : "r"((int)p), "l"(addr));
 }
 
 // ---- TMA (1-D bulk copy global -> shared) signalled on an mbarrier ----
@@ -1103,13 +1086,6 @@ extern "C" __global__ void __launch_bounds__(SPEC_BLOCK, SPEC_MIN_BLOCKS)
                 index = max(ra, rb);
             }
             const bool defer = (m & PU_ALWAYS_DEFERS) || ((m & PU_MISS_DEFERS) && index < 0);
-#if SPEC_PRED && !SPEC_HIST && !SPEC_INFO
-            {
-                const bool settled = (m & PM_INRANGE) && !defer;
-                pred_red_add1(counts + max(index, 0), settled && index >= 0);
-                if (SPEC_HAS_INDEX) pred_stcs(out_index + pend.i, index, settled);
-            }
-#else
             if ((m & PM_INRANGE) && !defer) {
                 if (index >= 0) count_hit(counts, hist_saddr, index);
                 if (SPEC_HAS_INDEX) __stcs(out_index + pend.i, index);
@@ -1117,7 +1093,6 @@ extern "C" __global__ void __launch_bounds__(SPEC_BLOCK, SPEC_MIN_BLOCKS)
                     __stcs(out_info + pend.i, pack_info(index >= 0, (m & PM_REV) != 0, (int)((m >> 16) & 0xFFu), 0, (int)(m & 0xFFFFu)));
                 }
             }
-#endif
             const uint32_t dm = __ballot_sync(0xFFFFFFFFu, defer);
             if (dm) {
                 if (defer) {
@@ -1145,16 +1120,6 @@ extern "C" __global__ void __launch_bounds__(SPEC_BLOCK, SPEC_MIN_BLOCKS)
 #if SPEC_JOINT
         // one table for both strands: the strand is bit 31 of the H word, the homes are the top bits of two multiply-adds
         pend.kh = kh + ((meta & PM_REV) ? 0x80000000u : 0u);
-#if SPEC_PRED
-        {
-            const bool probe = (meta & PM_CAND) && kn == 0;
-            const uint32_t x = joint_hash(pend.kh, kl);
-            const uint32_t second = (1u << (32 - tb.joint_shift)) + (joint_hash2(x) >> tb.joint_shift);
-            pred_ldcg(pend.a, tb.joint + (x >> tb.joint_shift), probe);
-            pred_ldcg(pend.b, tb.joint + second, probe);
-            pend.meta = meta + (probe ? PM_PROBED : 0u);
-        }
-#else
         if ((meta & PM_CAND) && kn == 0) {
             const uint32_t x = joint_hash(pend.kh, kl);
             const uint32_t second = (1u << (32 - tb.joint_shift)) + (joint_hash2(x) >> tb.joint_shift);
@@ -1163,7 +1128,6 @@ extern "C" __global__ void __launch_bounds__(SPEC_BLOCK, SPEC_MIN_BLOCKS)
             pend.b = __ldcg(tb.joint + second);
             pend.meta = meta + PM_PROBED;
         }
-#endif
 #else
         pend.kh = kh;
         if ((meta & PM_CAND) && kn == 0) {

@@ -226,23 +226,3 @@ def test_paired_and_random_designs_read_block_gzip(gpu, kref, monkeypatch):
             assert len(got) == len(want)
             for a, b in zip(want, got):
                 assert np.array_equal(np.asarray(a), np.asarray(b))
-
-
-@pytest.mark.parametrize("env", [{"SCG_INFLATE_ROUTE": "split", "SCG_INFLATE_WARP_FIRST": "0"},
-                                 {"SCG_INFLATE_ROUTE": "split", "SCG_INFLATE_WARP_FIRST": "0", "SCG_INFLATE_LIT_BITS": "10"},
-                                 {"SCG_INFLATE_LANES": "16"}, {"SCG_INFLATE_LANES": "8"}],
-                         ids=["lane_per_member", "lane_per_member_10_bit_tables", "16_lanes_per_member", "8_lanes_per_member"])
-def test_the_other_inflate_routes(env):
-    """The inflater's other routes (csrc/inflate.cu: one LANE per member decoding into symbols + one warp per member placing them;
-    two or four members per warp) are chosen once per process: this module's tests run again under each, in a process of their own."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get("SCG_TEST_INFLATE_ROUTES_INNER"):
-        pytest.skip("already inside the re-run")
-    child = dict(os.environ, SCG_TEST_INFLATE_ROUTES_INNER="1", **env)
-    here = os.path.dirname(os.path.abspath(__file__))
-    run = subprocess.run([sys.executable, "-m", "pytest", os.path.join(here, "test_gpu_bgzf.py"), "-x", "-q", "-m", "gpu", "-p", "no:cacheprovider"],
-                         env=child, cwd=os.path.dirname(here), capture_output=True, text=True, timeout=900)
-    assert run.returncode == 0, run.stdout[-3000:] + run.stderr[-2000:]
-    assert " passed" in run.stdout
